@@ -22,6 +22,10 @@ Every rank integrates the members `ebm.member_deal` hands it: 32-member packets 
 initial regime (a contiguous cut gives one rank all the expensive members; round-1 VERDICT).
 
 `--impl reference` times that CPU implementation alone (rank 0 only).
+
+`--dump-outputs DIR` writes what the last timed step of the headline pass (and of the MIZ sub-record) returned, for a
+fixed seeded sample of members, so that two builds of the project can be compared output for output: the inputs are
+the same from run to run for the same arguments.  Sampled members whose outputs are not finite are left out.
 """
 from __future__ import annotations
 
@@ -61,7 +65,14 @@ def parse():
     ap.add_argument("--no-extra", action="store_true", help="skip the strong-scaling and MIZ sub-records")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (diagnostics, final state, flags) "
+                         "for a fixed seeded sample of members as DIR/<workload>_<name>.npy, float64, under 64 MB in all "
+                         "(rank 0's members only; members with non-finite outputs left out)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ----------------------------------------------------------------------------- workloads
@@ -289,9 +300,10 @@ class Env:
         self.torch.cuda.synchronize()
 
 
-def device_pass(env, workload, nmem_total, years, steps, warmup, sample_clocks=False):
+def device_pass(env, workload, nmem_total, years, steps, warmup, sample_clocks=False, dump_dir=None, dump_bytes=0):
     """W warm-up + K timed steps of one workload; every rank integrates the members `member_deal` hands it.
-    Returns the measurements (max over ranks where it is a time) and what the e2e / CPU legs need."""
+    Returns the measurements (max over ranks where it is a time) and what the e2e / CPU legs need.  With `dump_dir`,
+    rank 0 writes a sample of the last timed step's outputs there (dump_outputs)."""
     torch, dist, ebm, _lib, lib, dev = env.torch, env.dist, env.ebm, env._lib, env.lib, env.dev
     world, rank = env.world, env.rank
     key = classic_cost_key(nmem_total) if workload == "classic" else None
@@ -358,6 +370,13 @@ def device_pass(env, workload, nmem_total, years, steps, warmup, sample_clocks=F
     env.barrier()
     launches = lib.ebm_launch_count() - launches0
     clocks = sampler.stop() if sampler else None
+    if dump_dir is not None and rank == 0:
+        if workload == "classic":
+            outs = {"diag": d_diag, "E_final": d_state[0].T, "Tg_final": d_state[1].T, "flags": d_flags}
+        else:
+            outs = {"diag": d_diag, **{f"{v}_final": t.T for v, t in zip(("Ei", "Ew", "h", "D", "phi", "T0"), d_state)},
+                    "newton_iters": d_i64[0], "nonconv": d_i64[1], "flags": d_flags}
+        dump_outputs(dump_dir, workload, mine, outs, dump_bytes)
     ms_total = t0.elapsed_time(t1)
     k_ms = float(np.mean([a.elapsed_time(b) for a, b in kern_ev]))
     k_all = [k_ms]
@@ -385,6 +404,30 @@ def device_pass(env, workload, nmem_total, years, steps, warmup, sample_clocks=F
            "mean_T_last_year_member0": float(d_diag[0, -1, 2, 0].item()) if nmem else None}
     res["_e2e_inputs"] = (st, par, forc, init, nmem)
     return res
+
+
+DUMP_BYTES = {"headline": 44_000_000, "miz": 16_000_000}   # under 64 MB in all, .npy headers included
+
+
+def dump_outputs(out_dir, workload, mine, outs, max_bytes):
+    """Write `outs` (name -> device tensor, member index first) for a sample of this rank's members as
+    out_dir/<workload>_<name>.npy in float64, plus <workload>_member_index.npy (global member indices of the rows).
+    The sample is drawn with a fixed seed from the member count alone and sized to `max_bytes`, so two builds of the
+    project run with the same arguments sample the same members.  Sampled members with a non-finite value in any
+    output are left out (members of the MIZ sweep whose state blows up, as it does in the reference algorithm; the
+    JSON line counts them as nan_members), so every value written is finite and comparable."""
+    import torch
+    nmem = len(mine)
+    per_member = 8 * (1 + sum(int(np.prod(t.shape[1:])) for t in outs.values()))
+    count = max(1, min(nmem, max_bytes // per_member))
+    pos = np.sort(np.random.default_rng(0).choice(nmem, size=count, replace=False))
+    sel = {name: t.index_select(0, torch.from_numpy(pos).to(t.device)) for name, t in outs.items()}
+    finite = torch.stack([torch.isfinite(s.reshape(count, -1)).all(dim=1) for s in sel.values()]).all(dim=0).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{workload}_member_index.npy"),
+            np.asarray(mine, dtype=np.int64)[pos[finite]].astype(np.float64))
+    for name, s in sel.items():
+        np.save(os.path.join(out_dir, f"{workload}_{name}.npy"), s.cpu().numpy()[finite].astype(np.float64))
 
 
 def roofline_record(env, workload, res, traffic):
@@ -428,7 +471,8 @@ def main():
     traffic = _traffic()
 
     # ---- headline: K timed steps of the requested workload, weak scaling (nmem members per GPU)
-    res = device_pass(env, args.workload, total, years, args.steps, args.warmup, sample_clocks=True)
+    res = device_pass(env, args.workload, total, years, args.steps, args.warmup, sample_clocks=True,
+                      dump_dir=args.dump_outputs, dump_bytes=DUMP_BYTES["headline"])
     roof = roofline_record(env, args.workload, res, traffic if (args.members == 0 and args.years == 0) else None)
     e2e = None
     if not args.no_e2e:
@@ -450,7 +494,8 @@ def main():
                       "kernel_ms_per_rank": sres["kernel_ms_per_rank"],
                       "note": "the fixed 65 536-member sweep (SURVEY 8e) dealt over the N ranks; NCCL gather inside the timed step"}
         mz_members, mz_years = args.miz_members, args.miz_years
-        mres = device_pass(env, "miz", mz_members * world, mz_years, min(args.steps, 3), 1)
+        mres = device_pass(env, "miz", mz_members * world, mz_years, min(args.steps, 3), 1,
+                           dump_dir=args.dump_outputs, dump_bytes=DUMP_BYTES["miz"])
         mroof = roofline_record(env, "miz", mres, traffic)
         me2e = None if args.no_e2e else run_e2e(env, "miz", mres["_e2e_inputs"], mz_years, mz_members * world)
         mcpu = cpu_baseline("miz", mz_members * world, mz_years, host_threads()) if (rank == 0 and not args.no_cpu) else None

@@ -9,6 +9,7 @@ from __future__ import annotations
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -24,10 +25,15 @@ _llp = ctypes.POINTER(ctypes.c_longlong)
 
 
 def build(force: bool = False) -> str:
-    """Compile the oracle with the committed Makefile (gcc, -ffp-contract=off)."""
+    """Compile the oracle with the committed Makefile (gcc, -ffp-contract=off).  In a read-only tree an out-of-date
+    library is compiled into a temporary directory instead."""
     src = os.path.join(_HERE, "ebm_oracle.c")
     if force or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src):
-        subprocess.run(["make", "-C", _HERE, "CC=gcc"], check=True, capture_output=True)
+        out_dir = os.path.dirname(_SO)
+        writable = os.access(out_dir if os.path.isdir(out_dir) else _HERE, os.W_OK)
+        out = _SO if writable else os.path.join(tempfile.mkdtemp(prefix="ebm_oracle_"), os.path.basename(_SO))
+        subprocess.run(["make", "-C", _HERE, "CC=gcc", f"OUT={out}"], check=True, capture_output=True)
+        return out
     return _SO
 
 
