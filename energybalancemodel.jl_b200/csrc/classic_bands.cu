@@ -1,6 +1,6 @@
 // classic_bands.cu -- band kernel of the classic (Wagner-Eisenman) EBM ensemble: the first fast kernel of this
-// library, now the fallback for grids with 208 < nx <= 256 (and EBM_CLASSIC_VARIANT < 0 / 11 for comparison);
-// classic_uniform.cu integrates everything up to 208 cells 2-3x faster.
+// library, now the kernel for grids with 208 < nx <= 256; classic_uniform.cu integrates everything up to 208 cells
+// 2-3x faster.
 //
 // Replaces, for a whole ensemble and many years per launch, the reference's
 //   integrate loop           src/infrastructure.jl:630-634
@@ -55,7 +55,6 @@ __global__ void __launch_bounds__(MAXT, MINB) classic_bands_kernel(const Classic
   const int band = band_raw < W ? band_raw : W - 1;   // (the launcher rounds W up to whole warps: band_raw < W always)
   const long long m_raw = (long long)blockIdx.x * MW + mi;
   const bool active = m_raw < a.nmem && band_raw < W;
-  if (a.uniform_split && ebm_classic_group_uniform<MW>(a.par, a.nmem, (long long)blockIdx.x * MW, mi)) return;
   const long long m = active ? m_raw : a.nmem - 1;
   const long long nmem = a.nmem;
   const int nx = a.nx, nt = a.nt;
@@ -353,9 +352,8 @@ int launch_variant(const ClassicKArgs& a0, cudaStream_t stream) {
 }  // namespace
 
 int ebm_launch_classic_bands(const ClassicKArgs& a, cudaStream_t stream) {
-  // K = cells per thread.  nx <= 130: 13 cells x up to 10 bands; larger grids use wider bands.
+  // up to 16 bands of 16 cells, 16 members per CTA
   if (a.nx <= 2) { ebm_set_error("classic_bands: nx must be > 2"); return EBM_ERR_INVALID; }
-  if (a.nx <= 100) return launch_variant<10, 32, 320, 1>(a, stream);
   if (a.nx <= 256) return launch_variant<16, 16, 256, 1>(a, stream);
   ebm_set_error("classic_bands: nx=%d > 256 not supported by the register-resident kernel", a.nx);
   return EBM_ERR_UNSUPPORTED;

@@ -1,8 +1,10 @@
 // classic_uniform.cu -- the classic (Wagner-Eisenman) EBM ensemble kernel for grids up to 208 cells.
 //
-// Two instances share this source: TAB = true integrates the 32-member groups whose table-building parameters
-// (D, cg, tau, S0, S2, a0, a2) agree -- forcing sweeps, hysteresis runs, sweeps over A, B, cw, S1, ai, Fb, k, Lf;
-// TAB = false the groups where they differ (coefficients applied per member, no precomputed pivots).
+// TAB = true integrates the 32-member groups whose table-building parameters (D, cg, tau, S0, S2, a0, a2) agree --
+// forcing sweeps, hysteresis runs, sweeps over A, B, cw, S1, ai, Fb, k, Lf; TAB = false the groups where they differ
+// (coefficients applied per member, no precomputed pivots).  UPAR = true (with TAB) takes a launch in which every
+// member has the same 15 parameters (the C4 forcing sweep).  Five instances: TAB, !TAB and UPAR with 8 bands for
+// nx <= 104, TAB and !TAB with 16 bands (255 registers, 1 CTA per SM) for 104 < nx <= 208.
 //
 // Mapping (B200 facts measured with scripts/microbench/fp64_lat.cu: DFMA latency 8.8 cycles, one warp can issue
 // a DFMA every 2.4 cycles, the 64 KB register file of an SM sub-partition holds 3 warps at <=168 registers):
@@ -51,22 +53,12 @@ constexpr double kTwoPi = 6.283185307179586;
 
 // reciprocal for well-scaled operands: MUFU.RCP64H seed + one cubic step (~1 ulp, no slow path)
 __device__ __forceinline__ double fast_rcp(double w) {
-#ifdef EBM_RCP_NEWTON2
-  double x;
-  asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(x) : "d"(w));
-  double e = fma(-w, x, 1.0);
-  x = fma(x, e, x);
-  e = fma(-w, x, 1.0);
-  x = fma(x, e, x);
-  return x;
-#else
   // the seed is good to 2^-20 (measured, profiles/r2_microbench.txt): one cubic step reaches 1 ulp
   double x;
   asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(x) : "d"(w));
   const double e = fma(-w, x, 1.0);
   const double t = fma(e, e, e);
   return fma(x, t, x);
-#endif
 }
 // sign tests on the high word (integer pipe, not the FP64 pipe).  The state never holds -0.0: it is normalised when
 // loaded, and E + dt*(...) cannot produce it (an exact cancellation rounds to +0.0).
@@ -77,27 +69,20 @@ struct __align__(16) PhysTab { double S0x, S1x, aw, wts; };      // per cell
 struct __align__(16) ElimTab { double iw, tq, q, s; };           // per row: band-local no-mask elimination
 struct __align__(16) CoefTab { double kjj, aoff, coff, ac; };    // per cell, masked path: ac = aoff_j * coff_{j-1} (0 on a band's first row)
 
-// rows of the band system that survive from the elimination to the back substitution: registers (QS_SMEM = false)
-// or thread-private shared memory [2K][threads] (conflict free), which frees 4K registers for more resident CTAs
-template <int K, bool QS_SMEM>
+// rows of the band system that survive from the elimination to the back substitution, in thread-private shared
+// memory [3K][threads] (conflict free), which frees 6K registers for more resident CTAs (DESIGN.md 4.1)
+template <int K>
 struct RowStore {
-  double q_[QS_SMEM ? 1 : K], s_[QS_SMEM ? 1 : K], r_[QS_SMEM ? 1 : K];
   double* base;
   int stride;
   // r(i) = E_i / (M E_i - kLf) = 1/(M - kLf/E_i) of the cell's CURRENT enthalpy, carried from step to step: this
   // step's T0 = C/(M - kLf/E) (classic.jl:50) is C*r of the previous step's update (:56-62 computes it anyway)
-  __device__ __forceinline__ double& r(int i) {
-    if constexpr (QS_SMEM) return base[(2 * K + i) * stride]; else return r_[i];
-  }
-  __device__ __forceinline__ double& q(int i) {
-    if constexpr (QS_SMEM) return base[(2 * i) * stride]; else return q_[i];
-  }
-  __device__ __forceinline__ double& s(int i) {
-    if constexpr (QS_SMEM) return base[(2 * i + 1) * stride]; else return s_[i];
-  }
+  __device__ __forceinline__ double& r(int i) { return base[(2 * K + i) * stride]; }
+  __device__ __forceinline__ double& q(int i) { return base[(2 * i) * stride]; }
+  __device__ __forceinline__ double& s(int i) { return base[(2 * i + 1) * stride]; }
 };
 
-template <int K, int WB, int MW, bool QS_SMEM, bool WARPM, bool TAB, bool UPAR>
+template <int K, int WB, int MW, bool TAB, bool UPAR>
 struct Ctx {
   static constexpr int NXP = K * WB;
   // tables / scratch in shared memory
@@ -134,9 +119,8 @@ struct Ctx {
   (void)dttau_cw; (void)dc; (void)inv_nt; (void)inv_Lf
   // thread identity
   int band, mi, j0;
-  // index of cell i of this thread in the per-cell shared arrays (annual sums): [cell][member] when a warp holds
-  // 16 members of 2 bands; thread-private [i][thread] (conflict free) when a warp holds all bands of 4 members
-  __device__ __forceinline__ int cidx(int i) const { return WARPM ? (i * (WB * MW) + (int)threadIdx.x) : ((j0 + i) * MW + mi); }
+  // index of cell i of this thread in the per-cell shared arrays (annual sums): [cell][member]
+  __device__ __forceinline__ int cidx(int i) const { return (j0 + i) * MW + mi; }
   bool active, sel, cta_fields;
   bool solver;   // this warp solves the CTA's interface systems (the warp that owns band pair 1: never the polar pair)
   // original member index of this thread's member (output rows, field selection): recomputed where it is needed (the
@@ -148,7 +132,7 @@ struct Ctx {
   }
   // state
   double E[K], Tg[K], accT;
-  RowStore<K, QS_SMEM> rs;
+  RowStore<K> rs;
   double* sumE;   // [NXP][MW] running annual sum of E per cell (shared memory: keeps 2K registers free)
 
   // annual sums and (SLOW only) sampled output of cell i after its update: savesol! (infrastructure.jl:549-591)
@@ -220,14 +204,8 @@ struct Ctx {
     }
   }
 
-#ifndef EBM_GI_UPAR
-#define EBM_GI_UPAR 5
-#endif
-#ifndef EBM_GIM_UPAR
-#define EBM_GIM_UPAR 4
-#endif
-  static constexpr int GI = UPAR ? EBM_GI_UPAR : 3;      // cells per statement-major group: all-ice path
-  static constexpr int GIM = UPAR ? EBM_GIM_UPAR : 3;    // mixed ice / water path
+  static constexpr int GI = UPAR ? 5 : 3;    // cells per statement-major group: all-ice path
+  static constexpr int GIM = UPAR ? 4 : 3;   // mixed ice / water path
   template <int I0, bool MIXED, bool SLOW>
   __device__ __forceinline__ void ice_group(const ClassicKArgs& a, const double fmA, const double S1c0, const double S1c1,
                                             const int season, const int ti, const int year, bool& anymask,
@@ -488,54 +466,9 @@ struct Ctx {
       i_sl = rs.s(K - 1); i_ql = rs.q(K - 1); i_yl = Tg[K - 1];
       i_al = al; i_be = be; i_ga = ga;
     }
-    double xL, xn;
-    if constexpr (WARPM) {
-      // ---- all WB bands of a member sit in one warp (lane = band * MPW + member): the interface system
-      //   A z_{b-1} + z_b + C z_{b+1} = R   is solved by parallel cyclic reduction over shuffles; no CTA barrier
-      constexpr int MPW = 32 / WB;                           // members per warp
-      constexpr unsigned kFull = 0xffffffffu;
-      const double nal = __shfl_down_sync(kFull, i_al, MPW), nbe = __shfl_down_sync(kFull, i_be, MPW);
-      const double nga = __shfl_down_sync(kFull, i_ga, MPW);
-      const double ql = (band == WB - 1) ? 0.0 : i_ql;
-      double A = (band == 0) ? 0.0 : i_sl;
-      double C = -ql * nga;
-      double R = fma(-ql, nal, i_yl);
-      {
-        const double ib = fast_rcp(fma(-ql, nbe, 1.0));
-        A *= ib; C *= ib; R *= ib;
-      }
-#pragma unroll
-      for (int st = 1; st < WB; st <<= 1) {
-        const double Au = __shfl_up_sync(kFull, A, st * MPW), Cu = __shfl_up_sync(kFull, C, st * MPW);
-        const double Ru = __shfl_up_sync(kFull, R, st * MPW);
-        const double Ad = __shfl_down_sync(kFull, A, st * MPW), Cd = __shfl_down_sync(kFull, C, st * MPW);
-        const double Rd = __shfl_down_sync(kFull, R, st * MPW);
-        const double a_ = (band >= st) ? A : 0.0, c_ = (band + st < WB) ? C : 0.0;
-        const double ib = fast_rcp(fma(-a_, Cu, fma(-c_, Ad, 1.0)));
-        const double Rn = fma(-a_, Ru, fma(-c_, Rd, R));
-        A = -(a_ * Au) * ib;
-        C = -(c_ * Cd) * ib;
-        R = Rn * ib;
-      }
-      xn = R;
-      const double zup = __shfl_up_sync(kFull, R, MPW);
-      xL = (band > 0) ? zup : 0.0;
-      if (SLOW && season >= 0) {                             // diagnostics: reduce the member's WB band partials
-#pragma unroll
-        for (int o = MPW; o < 32; o <<= 1) {
-          dgT += __shfl_xor_sync(kFull, dgT, o); dgE += __shfl_xor_sync(kFull, dgE, o);
-          dgA += __shfl_xor_sync(kFull, dgA, o); dgX = fmin(dgX, __shfl_xor_sync(kFull, dgX, o));
-        }
-        if (band == 0 && a.diag != nullptr && active) {
-          double* o = a.diag + ((member_orig(a) * a.dur + year) * 3 + season) * 4;
-          o[0] = dgT; o[1] = dgE; o[2] = kTwoPi * dgA; o[3] = (dgX > 1.5) ? 1.0 : dgX;
-        }
-      }
-      PHASE_MARK(3);
-    } else {
     {
-    double* f6 = iface + (band * 6) * MW + mi;
-    f6[0 * MW] = i_sl; f6[1 * MW] = i_ql; f6[2 * MW] = i_yl; f6[3 * MW] = i_al; f6[4 * MW] = i_be; f6[5 * MW] = i_ga;
+      double* f6 = iface + (band * 6) * MW + mi;
+      f6[0 * MW] = i_sl; f6[1 * MW] = i_ql; f6[2 * MW] = i_yl; f6[3 * MW] = i_al; f6[4 * MW] = i_be; f6[5 * MW] = i_ga;
     }
     if (SLOW && season >= 0) {
       double* r4 = red + (band * 4) * MW + mi;
@@ -600,9 +533,8 @@ struct Ctx {
     __syncthreads();
     PHASE_MARK(4);   // barrier 2 wait
     // ---- back substitution with the true neighbours
-    xL = (band > 0) ? zs[(band - 1) * MW + mi] : 0.0;
-    xn = zs[band * MW + mi];
-    }
+    const double xL = (band > 0) ? zs[(band - 1) * MW + mi] : 0.0;
+    double xn = zs[band * MW + mi];
     Tg[K - 1] = xn;
     if (!anymask) {
 #pragma unroll
@@ -623,34 +555,31 @@ struct Ctx {
   }
 };
 
-template <int K, int WB, int MW, bool QS_SMEM>
+template <int K, int WB, int MW>
 constexpr size_t uniform_smem_bytes(bool fields) {
   return (size_t)K * WB * (sizeof(PhysTab) + sizeof(ElimTab) + sizeof(CoefTab)) +
          sizeof(double) * ((size_t)2 * WB + (size_t)(WB + 1) * 6 * MW + (size_t)WB * MW * (1 + 4) + 10 * MW +
-                           (size_t)K * WB * MW + (fields ? (size_t)2 * K * WB * MW : 0) +
-                           (QS_SMEM ? (size_t)3 * K * WB * MW : 0));
+                           (size_t)K * WB * MW + (fields ? (size_t)2 * K * WB * MW : 0) + (size_t)3 * K * WB * MW);
 }
 
-template <int K, int WB, int MW, int MAXR, bool QS_SMEM, bool WARPM, bool TAB, bool UPAR>
+template <int K, int WB, int MW, int MAXR, bool TAB, bool UPAR>
 __global__ void __maxnreg__(MAXR) classic_uniform_kernel(const __grid_constant__ ClassicKArgs a) {
   static_assert(!UPAR || TAB, "launch-uniform parameters imply uniform tables");
   static_assert(MW == 16, "warp 0 = two lanes per member (full-warp shuffles)");
-  static_assert(!WARPM || (32 % WB == 0 && QS_SMEM), "member-in-warp mapping: WB bands x 32/WB members per warp");
   static_assert(WB % 2 == 0 && (WB * MW) % 32 == 0, "whole warps, even band count");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int BPW = 32 / MW;
   constexpr int NXP = K * WB;
   const int tid = threadIdx.x;
   const int lane = tid & 31, warp = tid >> 5;
-  // warp = BPW bands x MW members (interface through shared memory and two CTA barriers), or, WARPM, warp = all WB
-  // bands x 32/WB members (interface through shuffles, no barrier in the time loop)
-  const int mi = WARPM ? (warp * (32 / WB) + (lane & (32 / WB - 1))) : (lane & (MW - 1));
+  // warp = BPW bands x MW members (interface through shared memory and two CTA barriers)
+  const int mi = lane & (MW - 1);
   // which band pair a warp owns rotates with the CTA index: in a partially ice-covered member only the polar bands
   // take the expensive path, and without the rotation every resident CTA puts that warp on the same SM sub-partition
   constexpr int NWARP = WB * MW / 32;
   const unsigned bid = blockIdx.x + (unsigned)a.block0;   // 16-member group of this CTA
   const int wrot = (a.dbg & 4) ? warp : (int)((warp + bid) % NWARP);
-  const int band = WARPM ? (lane / (32 / WB)) : (wrot * BPW + lane / MW);
+  const int band = wrot * BPW + lane / MW;
   const long long nmem = a.nmem;
   const long long m_first = (long long)bid * MW;
   const long long m_raw = m_first + mi;
@@ -676,8 +605,8 @@ __global__ void __maxnreg__(MAXR) classic_uniform_kernel(const __grid_constant__
   double* red = zs + WB * MW;                                    // [WB][4][MW]
   double* fr = red + WB * 4 * MW;                                // [10][MW]
   double* sumE = fr + 10 * MW;                                   // [NXP][MW]
-  double* qsm = sumE + NXP * MW;                                 // [3K][threads] band rows q, s, r (QS_SMEM only)
-  double* sumT = qsm + (QS_SMEM ? 3 * NXP * MW : 0);             // [NXP][MW], only if the launch writes fields
+  double* qsm = sumE + NXP * MW;                                 // [3K][threads] band rows q, s, r
+  double* sumT = qsm + 3 * NXP * MW;                             // [NXP][MW], only if the launch writes fields
   double* sumH = sumT + NXP * MW;
 
   const double pD = par[0], pA = par[1], pB = par[2], pcw = par[3], pS0 = par[4], pS1 = par[5], pS2 = par[6];
@@ -734,7 +663,7 @@ __global__ void __maxnreg__(MAXR) classic_uniform_kernel(const __grid_constant__
     bandc[2 * b] = be; bandc[2 * b + 1] = ga;
   }
 
-  Ctx<K, WB, MW, QS_SMEM, WARPM, TAB, UPAR> cx;
+  Ctx<K, WB, MW, TAB, UPAR> cx;
   cx.S0m = pS0; cx.S2m = pS2; cx.a0m = pa0; cx.a2m = pa2; cx.facm = fac; cx.fac2m = fac * fac; cx.one_dttaum = one_dttau;
   cx.rs.base = qsm + tid;
   cx.rs.stride = WB * MW;
@@ -745,7 +674,7 @@ __global__ void __maxnreg__(MAXR) classic_uniform_kernel(const __grid_constant__
   cx.inv_nt_ = 1.0 / nt; cx.inv_Lf_ = 1.0 / pLf;
   const double cM = UPAR ? a.u.M : cx.M_, ckLf = UPAR ? a.u.kLf : cx.kLf_;
   cx.band = band; cx.mi = mi; cx.j0 = band * K;
-  cx.solver = WARPM ? false : ((a.dbg & 8) ? warp == 0 : (wrot == (NWARP > 1 ? 1 : 0)));
+  cx.solver = (a.dbg & 8) ? warp == 0 : (wrot == (NWARP > 1 ? 1 : 0));
   cx.active = active;
   const long long mo = a.orig != nullptr ? a.orig[m] : m;   // ebm_classic_device_args_t.member_index
   cx.sel = active && a.field_stride > 0 && (mo % a.field_stride) == 0;
@@ -811,15 +740,15 @@ __global__ void __maxnreg__(MAXR) classic_uniform_kernel(const __grid_constant__
   if (bad && a.flags != nullptr) atomicOr(a.flags + mo, 1);
 }
 
-template <int K, int WB, int MW, int MAXR, bool QS_SMEM = false, bool WARPM = false, bool TAB = true, bool UPAR = false>
+template <int K, int WB, int MW, int MAXR, bool TAB = true, bool UPAR = false>
 int launch_uniform(const ClassicKArgs& a, cudaStream_t stream) {
   if (a.nx > K * WB) {
     ebm_set_error("classic_uniform: nx=%d exceeds %d bands of %d cells", a.nx, WB, K);
     return EBM_ERR_UNSUPPORTED;
   }
   const bool fields = a.seasonal != nullptr && a.field_stride > 0;
-  const size_t smem = uniform_smem_bytes<K, WB, MW, QS_SMEM>(fields);
-  auto kern = classic_uniform_kernel<K, WB, MW, MAXR, QS_SMEM, WARPM, TAB, UPAR>;
+  const size_t smem = uniform_smem_bytes<K, WB, MW>(fields);
+  auto kern = classic_uniform_kernel<K, WB, MW, MAXR, TAB, UPAR>;
   EBM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   // leave room for several CTAs per SM: ask for the largest shared-memory carve-out (L1 is hardly used)
   EBM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -833,35 +762,33 @@ int launch_uniform(const ClassicKArgs& a, cudaStream_t stream) {
 
 }  // namespace
 
-int ebm_classic_uniform_max_nx() { return 208; }   // 8 bands of 13 cells up to nx = 104, 16 bands up to 208
-
-// resident CTAs of the production instantiation (nx <= 104) on the current device
+// resident CTAs of the production instantiation (nx <= kClassic8BandMaxNx) on the current device
 int ebm_classic_uniform_slots() {
   int dev = 0, sms = 0, per_sm = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) { cudaGetLastError(); return 0; }
-#ifdef EBM_DEV_FAST_BUILD
-  auto kern = classic_uniform_kernel<13, 8, 16, 168, true, false, true, true>;
-#else
-  auto kern = classic_uniform_kernel<13, 8, 16, 168, true, false, true, false>;
-#endif
-  const size_t smem = uniform_smem_bytes<13, 8, 16, true>(false);
+  auto kern = classic_uniform_kernel<13, 8, 16, 168, true, false>;
+  const size_t smem = uniform_smem_bytes<13, 8, 16>(false);
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 8 * 16, smem) != cudaSuccess) { cudaGetLastError(); return 0; }
   return sms * per_sm;
 }
 
+// <K cells per thread, WB bands, MW members per CTA, max registers per thread>.  Up to kClassic8BandMaxNx: band rows
+// (pivots / spikes / carried reciprocals) in thread-private shared memory, 168 registers, 3 CTAs (12 warps) per SM;
+// larger grids: 16 bands, 8 warps per CTA, 1 CTA per SM.  The mappings measured and rejected are in DESIGN.md 4.1.
+int ebm_launch_classic_uniform(const ClassicKArgs& a, cudaStream_t stream) {
+  if (a.nx > kClassic8BandMaxNx) return launch_uniform<13, 16, 16, 255>(a, stream);
+  if (a.upar) return launch_uniform<13, 8, 16, 168, true, true>(a, stream);
+  return launch_uniform<13, 8, 16, 168>(a, stream);
+}
+
 // groups whose table-building parameters differ between members (e.g. a sweep over D): same mapping, coefficients
 // applied per member, every band eliminated in full
 int ebm_launch_classic_general(const ClassicKArgs& a, cudaStream_t stream) {
-  if (a.nx > ebm_classic_uniform_max_nx()) return EBM_OK;
-  if (a.upar && a.nx <= 104) return EBM_OK;   // the launch-uniform instance integrated every group
-#ifdef EBM_DEV_FAST_BUILD
-  return EBM_OK;
-#else
-  if (a.nx > 104) return launch_uniform<13, 16, 16, 255, true, false, false>(a, stream);
-  return launch_uniform<13, 8, 16, 168, true, false, false>(a, stream);
-#endif
+  if (a.upar) return EBM_OK;   // the launch-uniform instance integrated every group
+  if (a.nx > kClassic8BandMaxNx) return launch_uniform<13, 16, 16, 255, false>(a, stream);
+  return launch_uniform<13, 8, 16, 168, false>(a, stream);
 }
 
 // dev: read and reset the phase counters (zeros unless built with -DEBM_PHASE_TIMING)
@@ -874,28 +801,5 @@ extern "C" int ebm_debug_phase_cycles(unsigned long long* out64) {
 #else
   for (int i = 0; i < 64; ++i) out64[i] = 0;
   return 1;
-#endif
-}
-
-// variant: 0 = default.  Other values select alternative instantiations for tuning (env EBM_CLASSIC_VARIANT).
-int ebm_launch_classic_uniform(const ClassicKArgs& a, int variant, cudaStream_t stream) {
-  if (a.nx > ebm_classic_uniform_max_nx()) return EBM_OK;   // larger grids: the band kernel integrates every group
-#ifdef EBM_DEV_FAST_BUILD   // dev: only the launch-uniform instance (compile time)
-  return launch_uniform<13, 8, 16, 168, true, false, true, true>(a, stream);
-#else
-  if (a.nx > 104) return launch_uniform<13, 16, 16, 255, true>(a, stream);   // 16 bands, 8 warps per CTA, 1 CTA per SM
-  switch (variant) {
-    // <K cells/thread, WB bands, MW members/CTA, max registers/thread, band rows in smem, member-in-warp mapping>
-    // measured at 65 536 members x 20 years (member-years/s); the rejected ones stay selectable for re-measurement
-    case 5: return launch_uniform<13, 8, 16, 255>(a, stream);               // rows in registers, 2 CTAs/SM:   735 k
-    case 7: return launch_uniform<13, 8, 16, 255, true>(a, stream);         // rows in smem, 2 CTAs/SM:         704 k
-    case 8: return launch_uniform<7, 16, 16, 128, true>(a, stream);         // 16 bands of 7 cells, 16 warps/SM: 583 k
-    case 9: return launch_uniform<13, 8, 16, 168, true, true>(a, stream);   // member-in-warp, no CTA barrier:   717 k
-    // default: band rows (pivots / spikes / carried reciprocals) in thread-private shared memory, 168 registers,
-    // 3 CTAs (12 warps) per SM: 921 k
-    default:
-      if (a.upar) return launch_uniform<13, 8, 16, 168, true, false, true, true>(a, stream);
-      return launch_uniform<13, 8, 16, 168, true>(a, stream);
-  }
 #endif
 }

@@ -244,6 +244,16 @@ int download_transposed(double* host, double* stage, const double* src, long lon
 
 long long nsel_of(long long nmem, int stride) { return stride > 0 ? (nmem + stride - 1) / stride : 0; }
 
+// The classic kernels: the literal-order one on request; up to kClassicUniformMaxNx cells the table-driven kernel
+// (the 32-member groups whose table-building parameters agree) and its per-member-coefficient instance (the other
+// groups); larger grids the band kernel.
+int launch_classic(const ClassicKArgs& a, bool strict, cudaStream_t stream) {
+  if (strict) return ebm_launch_classic_strict(a, stream);
+  if (a.nx > kClassicUniformMaxNx) return ebm_launch_classic_bands(a, stream);
+  EBM_TRY(ebm_launch_classic_uniform(a, stream));
+  return ebm_launch_classic_general(a, stream);
+}
+
 }  // namespace
 
 extern "C" int32_t ebm_shutdown(void) {
@@ -310,13 +320,12 @@ extern "C" int32_t ebm_classic_run_device(const ebm_grid_t* grid, const ebm_clas
     a.hthr = (int)(bits >> 32);
   }
   const int ypl = opt.years_per_launch > 0 ? opt.years_per_launch : grid->dur;
-  static const int variant = getenv("EBM_CLASSIC_VARIANT") ? atoi(getenv("EBM_CLASSIC_VARIANT")) : 0;
   // ---- launch-uniform parameters (a forcing sweep such as C4: members differ in forcing and initial state only).  The
   // member constants then travel in the kernel argument block and are constant-bank operands of the FP64 instructions;
   // the 26 registers they otherwise occupy go to instruction-level parallelism (classic_uniform.cu, UPAR).  The host
   // derives them with the same IEEE expressions the kernels evaluate per member, so the results are bit-identical.
   DevBufs upar_bufs;
-  if (!opt.strict && variant == 0 && a.nx <= 104 && !getenv("EBM_NO_UPAR")) {
+  if (!opt.strict && a.nx <= kClassic8BandMaxNx && !getenv("EBM_NO_UPAR")) {
     double* dhead = nullptr; int* ddiff = nullptr;
     EBM_TRY(upar_bufs.alloc(&dhead, EBM_CLASSIC_NPAR));
     EBM_TRY(upar_bufs.alloc(&ddiff, 1));
@@ -341,23 +350,20 @@ extern "C" int32_t ebm_classic_run_device(const ebm_grid_t* grid, const ebm_clas
   // two waves, the second 15 % full.  Cut instead into 8 ranges of CTAs on 8 streams, each advancing in chunks of
   // years: whenever a range finishes a chunk its slots go to whichever range is waiting, and the makespan
   // approaches work / slots.  Results are bit-identical (a CTA's arithmetic does not depend on the launch shape).
-  if (!opt.strict && variant >= 0 && variant < 20 && a.nx <= 104 && !getenv("EBM_NO_WAVE_BALANCE")) {
+  if (!opt.strict && a.nx <= kClassic8BandMaxNx && !getenv("EBM_NO_WAVE_BALANCE")) {
     const long long blocks = (a.nmem + 15) / 16;
     const long long slots = ebm_classic_uniform_slots();
     const long long waves = slots > 0 ? (blocks + slots - 1) / slots : 0;
     if (slots > 0 && blocks > slots && blocks <= 12 * slots && grid->dur >= 8 &&
         (double)(waves * slots) > 1.08 * (double)blocks) {
-      constexpr int SMAX = 32;
-      static const int S = std::min(SMAX, std::max(1, getenv("EBM_WB_STREAMS") ? atoi(getenv("EBM_WB_STREAMS")) : 8));
-      static const int nchunk = std::max(1, getenv("EBM_WB_CHUNKS") ? atoi(getenv("EBM_WB_CHUNKS")) : 16);
+      constexpr int S = 8, nchunk = 16;   // measured flat between 4 x 20 and 16 x 40 (DESIGN.md)
       const int chunk = std::min(ypl, std::max(1, grid->dur / nchunk));
-      a.uniform_split = 1;
       cudaEvent_t fork;
       EBM_CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
       EBM_CUDA_TRY(cudaEventRecord(fork, stream));
       int rc = EBM_OK;
-      cudaStream_t aux[SMAX];
-      cudaEvent_t done[SMAX];
+      cudaStream_t aux[S];
+      cudaEvent_t done[S];
       int made = 0;
       for (; made < S && rc == EBM_OK; ++made) {
         if (cudaStreamCreateWithFlags(&aux[made], cudaStreamNonBlocking) != cudaSuccess ||
@@ -372,8 +378,7 @@ extern "C" int32_t ebm_classic_run_device(const ebm_grid_t* grid, const ebm_clas
           b.block0 = blocks * q / made;
           b.nblocks = blocks * (q + 1) / made - b.block0;
           if (b.nblocks <= 0) continue;
-          rc = ebm_launch_classic_uniform(b, variant, aux[q]);
-          if (rc == EBM_OK) rc = ebm_launch_classic_general(b, aux[q]);
+          rc = launch_classic(b, false, aux[q]);
         }
       }
       for (int q = 0; q < made; ++q) {   // join (and release: destruction is deferred until the work has drained)
@@ -389,27 +394,7 @@ extern "C" int32_t ebm_classic_run_device(const ebm_grid_t* grid, const ebm_clas
   for (int y0 = 0; y0 < grid->dur; y0 += ypl) {
     a.year0 = y0;
     a.nyears = (y0 + ypl <= grid->dur) ? ypl : grid->dur - y0;
-    if (opt.strict) {
-      EBM_TRY(ebm_launch_classic_strict(a, stream));
-    } else {
-      // parameter-uniform 32-member groups take the table-driven kernel, everything else the general one
-      // nx <= 104: the table-driven kernel takes the 32-member groups whose table-building parameters agree, its
-      // per-member-coefficient instance the others; larger grids (or EBM_CLASSIC_VARIANT < 0): the band kernel
-      a.uniform_split = (a.nx <= ebm_classic_uniform_max_nx() && variant >= 0) ? 1 : 0;
-      if (a.uniform_split && variant >= 20 && opt.classic_stencil == 0) {
-        // experimental one-barrier kernel (classic_fused.cu; EBM_CLASSIC_VARIANT >= 20): measured slower than the
-        // two-barrier kernel in every regime (DESIGN.md 4.1), kept for the record
-        EBM_TRY(ebm_launch_classic_fused(a, variant, stream));
-        EBM_TRY(ebm_launch_classic_fused_general(a, stream));
-      } else if (a.uniform_split) {
-        // the production kernel (classic_uniform.cu); EBM_CLASSIC_VARIANT = 1..11 select its tuning instantiations
-        EBM_TRY(ebm_launch_classic_uniform(a, variant, stream));
-        if (variant == 11) EBM_TRY(ebm_launch_classic_bands(a, stream));
-        else EBM_TRY(ebm_launch_classic_general(a, stream));
-      } else {
-        EBM_TRY(ebm_launch_classic_bands(a, stream));
-      }
-    }
+    EBM_TRY(launch_classic(a, opt.strict != 0, stream));
   }
   return EBM_OK;
 }
@@ -443,13 +428,12 @@ extern "C" int32_t ebm_classic_run(const ebm_grid_t* grid, int64_t nmem, const e
   // within a regime); the kernels write every output row at the member's original index (member_index).
   std::vector<long long> perm;
   long long* dperm = nullptr;
-  if (!opt.strict && nmem > 32 && !getenv("EBM_NO_REORDER")) {
+  if (!opt.strict && nmem > 32) {
     // primary key: the set of table-building parameters (D, S0, S2, a0, a2, cg, tau -- the table-driven kernel needs
     // them uniform over 32-member groups), numbered in order of first appearance; secondary: regime of the initial
     // state (0 ice free, 1 partial cover, 2 every cell ice).  Ensembles made of many distinct parameter sets
     // (a pure sweep over D) are left in the caller's order within each regime.
-    static const int kTablePar[7] = {0, 4, 6, 7, 8, 13, 14};
-    std::map<std::array<double, 7>, int> sets;
+    std::map<std::array<double, kClassicNTablePar>, int> sets;
     std::vector<int> key((size_t)nmem);
     const double* prow = (const double*)par;
     bool many_sets = false;
@@ -459,8 +443,8 @@ extern "C" int32_t ebm_classic_run(const ebm_grid_t* grid, int64_t nmem, const e
       const int regime = ice == 0 ? 0 : (ice == nx ? 2 : 1);
       int sid = 0;
       if (!many_sets) {
-        std::array<double, 7> tp;
-        for (int q = 0; q < 7; ++q) tp[q] = prow[m * EBM_CLASSIC_NPAR + kTablePar[q]];
+        std::array<double, kClassicNTablePar> tp;
+        for (int q = 0; q < kClassicNTablePar; ++q) tp[q] = prow[m * EBM_CLASSIC_NPAR + ebm_classic_table_par(q)];
         auto it = sets.find(tp);
         if (it == sets.end()) it = sets.emplace(tp, (int)sets.size()).first;
         sid = it->second;

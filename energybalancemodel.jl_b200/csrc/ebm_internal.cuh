@@ -66,14 +66,14 @@ struct ClassicKArgs {
   int year0, nyears;             // integrate years [year0, year0+nyears), 0-based
   int start_year;                // years already simulated before this run: added to the time passed to Forcing
   int winter_inx, summer_inx, lastonly, field_stride, all_const_forcing;
-  int uniform_split;             // 1: classic_uniform.cu integrates parameter-uniform 32-member groups, classic_bands.cu the rest
+  int reserved;                  // unused: keeps the argument-block layout, and with it the measured code of the classic kernels
   EbmGridTables g;
   const double* par;             // [15][nmem]
   const double* forc;            // [10][nmem]
   double* E; double* Tg;         // [nx][nmem]
   double* diag; double* seasonal; double* raw; int* flags;
   const long long* orig;         // NULL or [nmem]: original member index of slot m (output rows, field selection)
-  int dbg;                       // development switches (env EBM_DBG)
+  int dbg;                       // development switches (env EBM_DBG): 4 no band-pair rotation, 8 warp 0 solves the interface
   int hthr;                      // high word of 512/nt: an open-water cell with E above it cannot freeze within one step
   int upar;                      // 1: u is valid (every member of the launch shares all 15 parameters)
   ClassicUPar u;
@@ -98,12 +98,13 @@ struct MizKArgs {
 };
 
 // launchers (each returns an EBM_* status; kernels are enqueued on `stream`)
+// classic_uniform.cu integrates grids of up to 16 bands of 13 cells; up to 8 bands it runs 3 CTAs per SM and has
+// the launch-uniform-parameter instance.  Larger grids take classic_bands.cu.
+constexpr int kClassic8BandMaxNx = 13 * 8;
+constexpr int kClassicUniformMaxNx = 13 * 16;
 int ebm_launch_classic_bands(const ClassicKArgs& a, cudaStream_t stream);
-int ebm_launch_classic_uniform(const ClassicKArgs& a, int variant, cudaStream_t stream);
+int ebm_launch_classic_uniform(const ClassicKArgs& a, cudaStream_t stream);
 int ebm_launch_classic_general(const ClassicKArgs& a, cudaStream_t stream);
-int ebm_launch_classic_fused(const ClassicKArgs& a, int variant, cudaStream_t stream);          // classic_fused.cu
-int ebm_launch_classic_fused_general(const ClassicKArgs& a, cudaStream_t stream);
-int ebm_classic_uniform_max_nx();
 int ebm_classic_uniform_slots();   // resident CTAs of the production kernel on the current device (wave balancing)
 int ebm_launch_classic_strict(const ClassicKArgs& a, cudaStream_t stream);
 int ebm_launch_classic_single_step(const EbmGridTables& g, const double* par15, int ti, double f,
@@ -140,6 +141,15 @@ __device__ __forceinline__ double ebm_global_time(long long tinx, int nt) {
   return __ddiv_rn((double)(2 * tinx - 1), (double)(2LL * nt));
 }
 
+// The classic parameters that feed the CTA-wide tables of classic_uniform.cu: D, cg, tau (the matrix kappa,
+// classic.jl:21) and S0, S2, a0, a2 (insolation / albedo profiles, :23-28); A, B, cw, S1, ai, Fb, k, Lf are
+// per-member registers.
+constexpr int kClassicNTablePar = 7;
+__host__ __device__ constexpr int ebm_classic_table_par(int q) {
+  constexpr int k[kClassicNTablePar] = {0, 4, 6, 7, 8, 13, 14};
+  return k[q];
+}
+
 // Do the members of the 32-aligned group that contains this CTA's members share the table-building classic
 // parameters bit for bit?  Called by every thread of the CTA (contains a barrier); mi = member slot of the thread, MW = members per
 // CTA (a divisor of 32).  The uniform and the general kernel use this same rule to split an ensemble between them.
@@ -152,11 +162,8 @@ __device__ __forceinline__ bool ebm_classic_group_uniform(const double* __restri
   for (int r = 0; r < 32 / MW; ++r) {
     long long mm = g0 + mi + (long long)r * MW;
     if (mm >= nmem) mm = nmem - 1;
-    // only the parameters that feed the CTA-wide tables must agree: D, cg, tau (the matrix kappa, classic.jl:21) and
-    // S0, S2, a0, a2 (insolation / albedo profiles, :23-28); A, B, cw, S1, ai, Fb, k, Lf are per-member registers
-    constexpr int kTablePar[7] = {0, 4, 6, 7, 8, 13, 14};
-    for (int q = 0; q < 7; ++q) {
-      const int k = kTablePar[q];
+    for (int q = 0; q < kClassicNTablePar; ++q) {
+      const int k = ebm_classic_table_par(q);
       same = same && (par[(long long)k * nmem + mm] == par[(long long)k * nmem + g0]);
     }
   }

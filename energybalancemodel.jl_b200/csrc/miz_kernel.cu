@@ -8,7 +8,7 @@
 //   savesol! / annual_mean    src/infrastructure.jl:536-591
 // The literal-order twin of this kernel (bit-identical to the oracle) is miz_literal.cuh / miz_strict.cu; the
 // algebra here is the same step with
-//   * every division turned into a reciprocal (MUFU.RCP64H seed + 2 Newton steps) times a product, reciprocals
+//   * every division turned into a reciprocal (MUFU.RCP64H seed + one cubic step) times a product, reciprocals
 //     shared between quotients with the same denominator, constant quotients hoisted per member; denominators that
 //     the reference masks afterwards (zeroref!: D == 0, h == 0, n + dn == 0, phi == 1) are replaced by 1 BEFORE
 //     the reciprocal so that open-water cells never enter the IEEE slow path (they did 13 times per cell-step in the
@@ -28,7 +28,6 @@
 // Results agree with the oracle to rounding over short horizons; the MIZ dynamics amplify rounding differences
 // (DESIGN.md "MIZ sensitivity"), so long runs are compared through the literal kernel instead.
 #include <math.h>
-#include <stdlib.h>
 #include <type_traits>
 #include <string.h>
 
@@ -39,9 +38,7 @@ namespace {
 constexpr double kPi = 3.141592653589793;   // Float64(pi)
 constexpr unsigned kFull = 0xffffffffu;
 constexpr int kWarps = 4;                   // members per CTA
-#ifndef EBM_MIZ_GC
-#define EBM_MIZ_GC 3
-#endif
+constexpr int kGC = 3;                      // cells per statement-major group when K allows it (DESIGN.md 4.3)
 
 __device__ __forceinline__ double shfl_up1(double v) { return __shfl_up_sync(kFull, v, 1); }
 __device__ __forceinline__ double shfl_dn1(double v) { return __shfl_down_sync(kFull, v, 1); }
@@ -61,16 +58,8 @@ __device__ __forceinline__ double warp_min(double v) {
 __device__ __forceinline__ double rcp_nr(double y) {
   double r;
   asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(y));
-#ifdef EBM_MIZ_RCP_NEWTON2
-  double e = fma(-y, r, 1.0);
-  r = fma(r, e, r);
-  e = fma(-y, r, 1.0);
-  r = fma(r, e, r);
-  return r;
-#else
   const double e = fma(-y, r, 1.0);
   return fma(r, fma(e, e, e), r);
-#endif
 }
 // c ? a : b as one SELP with both operands evaluated: the compiler otherwise branches around "expensive" operands,
 // which splits the unrolled per-cell code into scheduling regions and serialises the K cells of a lane
@@ -81,10 +70,6 @@ __device__ __forceinline__ double keep(double v) {
   return v;
 }
 __device__ __forceinline__ double sel(bool c, double a, double b) { return c ? keep(a) : keep(b); }
-#ifdef EBM_MIZ_SELP
-__device__ __forceinline__ double sel0(bool c, double b) { return c ? 0.0 : keep(b); }   // c ? 0 : b
-__device__ __forceinline__ double sel1(bool c, double b) { return c ? 1.0 : keep(b); }   // c ? 1 : b
-#else
 // c ? 0 : b and c ? 1 : b as bit masks on the two words (2 LOP3 each; the mask of a condition is shared by all its
 // uses): ptxas lowers a select against an immediate 0.0 / 1.0 to "materialise the constant + two predicated moves",
 // 3-4 instructions per select and a third of this kernel's instruction count (profiles/r2_miz_fast_ncu.txt)
@@ -96,7 +81,6 @@ __device__ __forceinline__ double sel1(bool c, double b) {
   const int m = c ? 0 : -1;
   return __hiloint2double((__double2hiint(b) & m) | (0x3ff00000 & ~m), __double2loint(b) & m);
 }
-#endif
 // zero / sign tests on the integer pipe (the FP64 pipe is the bottleneck); +0 and -0 are both zero
 __device__ __forceinline__ bool is_zero(double v) { return ((__double2hiint(v) & 0x7fffffff) | __double2loint(v)) == 0; }   // one LOP3 with predicate output
 // x / y with y an ordinary non-zero number (no denormal / huge denominators: DESIGN.md 4.3)
@@ -446,7 +430,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
       // two instantiations: the hot one (no sampling this step, no field output) is straight-line code
       auto cells = [&](auto slow_tag) {
       constexpr bool SLOW = decltype(slow_tag)::value;
-      constexpr int GC = (K % EBM_MIZ_GC == 0) ? EBM_MIZ_GC : 2;   // cells per statement-major group (K is even)
+      constexpr int GC = (K % kGC == 0) ? kGC : 2;   // cells per statement-major group (K is even)
       // ptxas keeps the source order to a large extent and a warp issues in order: written cell after cell, the six
       // ~100-instruction dependent chains of a lane run one after the other (static schedule: 2.6 issue cycles per FP64
       // instruction).  Statement-major over groups of GC cells -- every statement for the group's cells before the
@@ -594,13 +578,7 @@ int ebm_launch_miz_fast(const MizKArgs& a, cudaStream_t stream) {
   if (a.single_ti > 0) return ebm_launch_miz_strict(a, stream);
   if (a.nx <= 64) return launch_k<2, 4>(a, stream);
   if (a.nx <= 128) return launch_k<4, 4>(a, stream);
-  if (a.nx <= 192) {
-    // resident CTAs per SM (register cap 255 / 168 / 128): tuning knob, default = fastest measured
-    static const int minb = getenv("EBM_MIZ_MINB") ? atoi(getenv("EBM_MIZ_MINB")) : 3;
-    if (minb == 2) return launch_k<6, 2>(a, stream);
-    if (minb == 4) return launch_k<6, 4>(a, stream);
-    return launch_k<6, 3>(a, stream);
-  }
+  if (a.nx <= 192) return launch_k<6, 3>(a, stream);   // 3 resident CTAs per SM (168 registers): fastest measured
   if (a.nx <= 256) return launch_k<8, 2>(a, stream);
   ebm_set_error("miz: nx=%d > 256 not supported by the register-resident kernel", a.nx);
   return EBM_ERR_UNSUPPORTED;

@@ -1,7 +1,7 @@
 """Dev helper: error statistics of the fast classic kernel against the oracle on the parity-test ensembles, beside
 the oracle's own solver-to-solver difference (tridiagonal vs the reference's dense LU) on the same inputs.
 
-    EBM_CLASSIC_VARIANT=<v> python scripts/dev_classic_err.py
+    python scripts/dev_classic_err.py
 """
 import os
 import sys
@@ -36,7 +36,6 @@ def report(name, st, forcings, pars, inits, stride):
         print("   |E_ref| at the cells with err > 5e-10:", sorted({round(float(abs(Eref[a, b, d])), 4) for a, b, c, d in big})[:12])
 
 
-print("variant", os.environ.get("EBM_CLASSIC_VARIANT", "0"))
 for nmem, nx, nt in [(70, 100, 2000), (33, 60, 1000), (5, 37, 500)]:
     st = ebm.SpaceTime(nx, nt, 3)
     f, p, i = _ensemble(nmem, nx)

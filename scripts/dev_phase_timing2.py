@@ -1,5 +1,5 @@
 """dev: per-phase cycle breakdown of the classic kernel (CTA 0) at full residency (444 CTAs), by regime.
-run: EBM_CUDA_LIB=energybalancemodel.jl_b200/lib/libebm_dev_pt.so python scripts/dev_phase_timing2.py   (library: scripts/dev_variant_lib.sh pt -DEBM_PHASE_TIMING)"""
+run: EBM_CUDA_LIB=energybalancemodel.jl_b200/lib/libebm_cuda_pt.so python scripts/dev_phase_timing2.py   (library: scripts/dev_phase_timing.sh)"""
 import ctypes as C, sys, time
 sys.path.insert(0, ".")
 import numpy as np

@@ -6,7 +6,6 @@
 snow: cold start (every cell ice, stays a snowball), F = -20..+20; free: warm start, F = +14..+20 (ice free after the
 spin-up); partial: warm start, F = -8..+8 (seasonal / perennial polar ice); c4: the bench.py C4 mix.  The state is
 spun up for `--spinup` years first so that the timed launches see the regime's steady state.
-EBM_CLASSIC_VARIANT selects the kernel instantiation (read once per process).
 """
 from __future__ import annotations
 
@@ -38,7 +37,7 @@ def main():
     p = ebm.default_parameters("Classic")
     prow = np.array([p[k] for k in ebm.CLASSIC_PAR_ORDER])
     n = a.members
-    out = {"variant": os.environ.get("EBM_CLASSIC_VARIANT", "0"), "members": n, "years": a.years}
+    out = {"members": n, "years": a.years}
     for regime in a.regimes.split(","):
         m = np.arange(n)
         if regime == "snow":
