@@ -18,7 +18,6 @@
 // ----------------------------------------------------------------------------- errors / counters
 static thread_local char g_err[512] = "";
 static std::atomic<long long> g_launches{0};
-thread_local EbmDiagHook* ebm_tl_diag_hook = nullptr;
 
 void ebm_set_error(const char* fmt, ...) {
   va_list ap;
@@ -147,13 +146,6 @@ int get_tables(const ebm_grid_t* g, EbmGridTables* out, cudaStream_t stream) {
   return EBM_OK;
 }
 
-ebm_options_t default_options() {
-  ebm_options_t o;
-  memset(&o, 0, sizeof(o));
-  o.device = -1; o.lastonly = 1;
-  return o;
-}
-
 // Restores the caller's current CUDA device when an entry point returns (select_device may change it).
 struct DeviceRestore {
   int prev = -1;
@@ -229,8 +221,6 @@ struct StreamGuard {
   ~StreamGuard() { cudaStreamSynchronize(s); cudaStreamDestroy(s); cudaGetLastError(); }
 };
 
-#define EBM_TRY(expr) do { int _rc = (expr); if (_rc != EBM_OK) return _rc; } while (0)
-
 // host [rows][cols] -> device [cols][rows] via a staging buffer
 int upload_transposed(const double* host, double* stage, double* dst, long long rows, long long cols, cudaStream_t s) {
   EBM_CUDA_TRY(cudaMemcpyAsync(stage, host, sizeof(double) * rows * cols, cudaMemcpyHostToDevice, s));
@@ -254,7 +244,203 @@ int launch_classic(const ClassicKArgs& a, bool strict, cudaStream_t stream) {
   return ebm_launch_classic_general(a, stream);
 }
 
+// The opening steps of ebm_classic_run_device and ebm_miz_run_device after their pointer checks: device, the
+// field-output check, the grid tables and the argument-block fields both models name alike.  The caller holds the
+// DeviceRestore.
+template <typename KArgs, typename DeviceArgs>
+int device_prologue(const ebm_grid_t* grid, const DeviceArgs* args, const ebm_options_t& opt, KArgs* a,
+                    cudaStream_t stream) {
+  if (args->nmem < 1) { ebm_set_error("nmem must be >= 1"); return EBM_ERR_INVALID; }
+  EBM_TRY(select_device(opt));
+  if ((args->seasonal || args->raw) && opt.field_stride <= 0) { ebm_set_error("seasonal/raw output requested but field_stride == 0"); return EBM_ERR_INVALID; }
+  memset(a, 0, sizeof(*a));
+  EBM_TRY(get_tables(grid, &a->g, stream));
+  a->nx = grid->nx; a->nt = grid->nt; a->dur = grid->dur; a->nmem = args->nmem;
+  a->winter_inx = grid->winter_inx; a->summer_inx = grid->summer_inx;
+  a->lastonly = opt.lastonly; a->field_stride = opt.field_stride;
+  a->start_year = opt.start_year > 0 ? opt.start_year : 0;
+  return EBM_OK;
+}
+
+// the run in launches of opt.years_per_launch years
+template <typename KArgs, typename Launch>
+int launch_years(KArgs a, const ebm_grid_t* grid, const ebm_options_t& opt, Launch launch) {
+  const int ypl = opt.years_per_launch > 0 ? opt.years_per_launch : grid->dur;
+  for (int y0 = 0; y0 < grid->dur; y0 += ypl) {
+    a.year0 = y0;
+    a.nyears = (y0 + ypl <= grid->dur) ? ypl : grid->dur - y0;
+    EBM_TRY(launch(a));
+  }
+  return EBM_OK;
+}
+
+// Lanes of a warp are members: members in different regimes (snowball next to ice free) make every warp take both code
+// paths.  Sort the members by the regime of their initial state (stable: the caller's order survives within a regime);
+// the kernels write every output row at the member's original index (member_index).
+std::vector<long long> classic_member_order(const ebm_grid_t* grid, long long nmem, const EbmHostRun& run,
+                                            const ebm_options_t& opt) {
+  std::vector<long long> perm;
+  if (opt.strict || nmem <= 32) return perm;
+  // primary key: the set of table-building parameters (D, S0, S2, a0, a2, cg, tau -- the table-driven kernel needs
+  // them uniform over 32-member groups), numbered in order of first appearance; secondary: regime of the initial
+  // state.  Ensembles made of many distinct parameter sets (a pure sweep over D) are left in the caller's order
+  // within each regime.
+  const int nx = grid->nx;
+  std::map<std::array<double, kClassicNTablePar>, int> sets;
+  std::vector<int> key((size_t)nmem);
+  bool many_sets = false;
+  for (long long m = 0; m < nmem; ++m) {
+    int sid = 0;
+    if (!many_sets) {
+      std::array<double, kClassicNTablePar> tp;
+      for (int q = 0; q < kClassicNTablePar; ++q) tp[q] = run.par[m * EBM_CLASSIC_NPAR + ebm_classic_table_par(q)];
+      auto it = sets.find(tp);
+      if (it == sets.end()) it = sets.emplace(tp, (int)sets.size()).first;
+      sid = it->second;
+      if ((long long)sets.size() * 32 > nmem) many_sets = true;   // groups cannot be made uniform anyway
+    }
+    key[m] = sid * 4 + ebm_classic_regime(run.init[0] + m * nx, nx);
+  }
+  if (many_sets) for (long long m = 0; m < nmem; ++m) key[m] &= 3;
+  if (std::is_sorted(key.begin(), key.end())) return perm;
+  perm.resize((size_t)nmem);
+  for (long long m = 0; m < nmem; ++m) perm[m] = m;
+  std::stable_sort(perm.begin(), perm.end(), [&](long long a, long long b) { return key[a] < key[b]; });
+  return perm;
+}
+
+// The per-model step of a host run: the public device entry point on the run's device arrays.
+int call_classic_device(const ebm_grid_t* grid, long long nmem, const EbmHostRun& dev, const long long* member_index,
+                        const ebm_options_t& opt, cudaStream_t stream) {
+  const ebm_classic_device_args_t da = {nmem, dev.par, dev.forc, dev.fin[0], dev.fin[1], dev.diag, dev.seasonal, dev.raw,
+                                        dev.flags, (const int64_t*)member_index};
+  return ebm_classic_run_device(grid, &da, &opt, stream);
+}
+
+int call_miz_device(const ebm_grid_t* grid, long long nmem, const EbmHostRun& dev, const long long*,
+                    const ebm_options_t& opt, cudaStream_t stream) {
+  const ebm_miz_device_args_t da = {nmem, dev.par, dev.forc, dev.fin[0], dev.fin[1], dev.fin[2], dev.fin[3], dev.fin[4],
+                                    dev.fin[5], dev.diag, dev.seasonal, dev.raw, dev.newton_iters, dev.nonconv, dev.flags};
+  return ebm_miz_run_device(grid, &da, &opt, stream);
+}
+
 }  // namespace
+
+// ----------------------------------------------------------------------------- host-buffer runs
+ebm_options_t default_options() {
+  ebm_options_t o;
+  memset(&o, 0, sizeof(o));
+  o.device = -1; o.lastonly = 1;
+  return o;
+}
+
+int ebm_classic_regime(const double* E, int nx) {
+  int ice = 0;
+  for (int j = 0; j < nx; ++j) ice += E[j] < 0.0;
+  return ice == 0 ? 0 : (ice == nx ? 2 : 1);
+}
+
+int ebm_run_host(const ebm_grid_t* grid, long long nmem, const EbmHostRun& run, const ebm_options_t* opt_in,
+                 EbmDiagHook* diag_hook) {
+  EBM_TRY(check_grid(grid));
+  ebm_options_t opt = opt_in ? *opt_in : default_options();
+  DeviceRestore _dr;
+  EBM_TRY(select_device(opt));
+  if ((run.seasonal || run.raw) && opt.field_stride <= 0) { ebm_set_error("seasonal/raw output requested but field_stride == 0"); return EBM_ERR_INVALID; }
+  const int nx = grid->nx, nt = grid->nt, dur = grid->dur;
+  const long long nsel = nsel_of(nmem, opt.field_stride);
+  const long long nraw = opt.lastonly ? nt : (long long)nt * dur;
+  const std::vector<long long> perm = run.order ? run.order(grid, nmem, run, opt) : std::vector<long long>();
+  cudaStream_t s;
+  EBM_CUDA_TRY(cudaStreamCreate(&s));
+  DevBufs B;                 // declared first: destroyed last
+  StreamGuard sg{s};         // ... after the stream has drained (error paths return without a synchronise of their own)
+  double *stage, *dpar, *dforc;
+  long long* dperm = nullptr;
+  EBM_TRY(B.alloc(&stage, (size_t)nmem * std::max(nx, run.npar)));
+  if (!perm.empty()) {
+    EBM_TRY(B.alloc(&dperm, (size_t)nmem));
+    EBM_CUDA_TRY(cudaMemcpyAsync(dperm, perm.data(), sizeof(long long) * nmem, cudaMemcpyHostToDevice, s));
+  }
+  auto upload = [&](const double* host, double* dst, long long cols) -> int {   // host [nmem][cols] -> device [cols][slots]
+    if (!dperm) return upload_transposed(host, stage, dst, nmem, cols, s);
+    EBM_CUDA_TRY(cudaMemcpyAsync(stage, host, sizeof(double) * nmem * cols, cudaMemcpyHostToDevice, s));
+    return ebm_launch_gather_transpose(stage, dst, nmem, cols, dperm, 0, s);
+  };
+  auto download = [&](double* host, const double* src) -> int {      // device [nx][slots] -> host [nmem][nx], original order
+    if (!dperm) return download_transposed(host, stage, src, nx, nmem, s);
+    EBM_TRY(ebm_launch_gather_transpose(src, stage, nmem, nx, dperm, 1, s));
+    EBM_CUDA_TRY(cudaMemcpyAsync(host, stage, sizeof(double) * nmem * nx, cudaMemcpyDeviceToHost, s));
+    return EBM_OK;
+  };
+  EbmHostRun dev = run;   // the same run on device arrays
+  EBM_TRY(B.alloc(&dpar, (size_t)nmem * run.npar));
+  EBM_TRY(B.alloc(&dforc, (size_t)nmem * EBM_NFORCING));
+  EBM_TRY(upload(run.par, dpar, run.npar));
+  EBM_TRY(upload(run.forc, dforc, EBM_NFORCING));
+  dev.par = dpar; dev.forc = dforc;
+  for (int q = 0; q < run.nstate; ++q) {
+    EBM_TRY(B.alloc(&dev.fin[q], (size_t)nmem * nx));
+    if (run.init[q]) EBM_TRY(upload(run.init[q], dev.fin[q], nx));
+    else EBM_CUDA_TRY(cudaMemsetAsync(dev.fin[q], 0, sizeof(double) * nmem * nx, s));
+    dev.init[q] = dev.fin[q];
+  }
+  // outputs: allocated when wanted; fields and diagnostics NaN (what the reference leaves undef), counters zero
+  const size_t ndiag = (size_t)nmem * dur * EBM_NSEASON * EBM_NDIAG;
+  const size_t nseas = (size_t)nsel * dur * EBM_NSEASON * run.nvar * nx;
+  const size_t nrawn = (size_t)nsel * nraw * run.nvar * nx;
+  auto nan_filled = [&](double** d, bool wanted, size_t n) -> int {
+    *d = nullptr;
+    if (!wanted) return EBM_OK;
+    EBM_TRY(B.alloc(d, n));
+    return ebm_launch_fill(*d, (long long)n, NAN, s);
+  };
+  auto zeroed = [&](auto** d, bool wanted) -> int {
+    *d = nullptr;
+    if (!wanted) return EBM_OK;
+    EBM_TRY(B.alloc(d, (size_t)nmem));
+    EBM_CUDA_TRY(cudaMemsetAsync(*d, 0, sizeof(**d) * nmem, s));
+    return EBM_OK;
+  };
+  EBM_TRY(nan_filled(&dev.diag, run.diag || diag_hook, ndiag));
+  EBM_TRY(nan_filled(&dev.seasonal, run.seasonal, nseas));
+  EBM_TRY(nan_filled(&dev.raw, run.raw, nrawn));
+  EBM_TRY(zeroed(&dev.newton_iters, run.newton_iters));
+  EBM_TRY(zeroed(&dev.nonconv, run.nonconv));
+  EBM_TRY(zeroed(&dev.flags, run.flags));
+  EBM_TRY(run.run_device(grid, nmem, dev, dperm, opt, s));
+  auto fetch = [&](auto* host, const auto* d, size_t n) -> int {
+    if (host) EBM_CUDA_TRY(cudaMemcpyAsync(host, d, sizeof(*host) * n, cudaMemcpyDeviceToHost, s));
+    return EBM_OK;
+  };
+  if (diag_hook) EBM_TRY(diag_hook->consume(dev.diag, ndiag, s));
+  else EBM_TRY(fetch(run.diag, dev.diag, ndiag));
+  EBM_TRY(fetch(run.seasonal, dev.seasonal, nseas));
+  EBM_TRY(fetch(run.raw, dev.raw, nrawn));
+  EBM_TRY(fetch(run.newton_iters, dev.newton_iters, (size_t)nmem));
+  EBM_TRY(fetch(run.nonconv, dev.nonconv, (size_t)nmem));
+  EBM_TRY(fetch(run.flags, dev.flags, (size_t)nmem));
+  for (int q = 0; q < run.nstate; ++q)
+    if (run.fin[q]) EBM_TRY(download(run.fin[q], dev.fin[q]));
+  EBM_CUDA_TRY(cudaStreamSynchronize(s));   // the copies above share the stream: one wait covers them all
+  return EBM_OK;
+}
+
+EbmHostRun ebm_classic_host_run(const ebm_classic_params_t* par, const ebm_forcing_t* forc, const double* E0,
+                                const double* Tg0, const ebm_classic_outputs_t* out) {
+  return {EBM_CLASSIC_NPAR, EBM_CLASSIC_NVAR, 2, (const double*)par, (const double*)forc, {E0, Tg0},
+          out->diag, out->seasonal, out->raw, {out->E_final, out->Tg_final}, nullptr, nullptr, out->flags,
+          call_classic_device, classic_member_order};
+}
+
+EbmHostRun ebm_miz_host_run(const ebm_miz_params_t* par, const ebm_forcing_t* forc, const double* Ei0, const double* Ew0,
+                            const double* h0, const double* D0, const double* phi0, const double* T0guess,
+                            const ebm_miz_outputs_t* out) {
+  return {EBM_MIZ_NPAR, EBM_MIZ_NVAR, 6, (const double*)par, (const double*)forc, {Ei0, Ew0, h0, D0, phi0, T0guess},
+          out->diag, out->seasonal, out->raw,
+          {out->Ei_final, out->Ew_final, out->h_final, out->D_final, out->phi_final, out->T0_final},
+          out->newton_iters, out->nonconv, out->flags, call_miz_device, nullptr};
+}
 
 extern "C" int32_t ebm_shutdown(void) {
   std::lock_guard<std::mutex> lk(g_cache_mu);
@@ -291,25 +477,17 @@ extern "C" int32_t ebm_classic_run_device(const ebm_grid_t* grid, const ebm_clas
   cudaStream_t stream = (cudaStream_t)stream_;
   EBM_TRY(check_grid(grid));
   if (!args || !args->par || !args->forc || !args->E || !args->Tg) { ebm_set_error("classic_run_device: par, forc, E, Tg must be non-NULL"); return EBM_ERR_INVALID; }
-  if (args->nmem < 1) { ebm_set_error("nmem must be >= 1"); return EBM_ERR_INVALID; }
-  ebm_options_t opt = opt_in ? *opt_in : default_options();
+  const ebm_options_t opt = opt_in ? *opt_in : default_options();
   DeviceRestore _dr;
-  EBM_TRY(select_device(opt));
-  if ((args->seasonal || args->raw) && opt.field_stride <= 0) { ebm_set_error("seasonal/raw output requested but field_stride == 0"); return EBM_ERR_INVALID; }
-  if (opt.step_limit > 0) { ebm_set_error("step_limit is only supported by the MIZ path"); return EBM_ERR_UNSUPPORTED; }
   ClassicKArgs a;
-  memset(&a, 0, sizeof(a));
-  EBM_TRY(get_tables(grid, &a.g, stream));
+  EBM_TRY(device_prologue(grid, args, opt, &a, stream));
+  if (opt.step_limit > 0) { ebm_set_error("step_limit is only supported by the MIZ path"); return EBM_ERR_UNSUPPORTED; }
   if (opt.classic_stencil == 1) {   // classic on non-uniform grids: the generic flux-form stencil in kappa
     a.g.lam_lo = a.g.glam_lo; a.g.lam_hi = a.g.glam_hi;
   } else if (opt.classic_stencil != 0) {
     ebm_set_error("classic_stencil must be 0 (get_diffop, as the reference) or 1 (generic flux-form stencil)");
     return EBM_ERR_INVALID;
   }
-  a.nx = grid->nx; a.nt = grid->nt; a.dur = grid->dur; a.nmem = args->nmem;
-  a.winter_inx = grid->winter_inx; a.summer_inx = grid->summer_inx;
-  a.lastonly = opt.lastonly; a.field_stride = opt.field_stride;
-  a.start_year = opt.start_year > 0 ? opt.start_year : 0;
   a.par = args->par; a.forc = args->forc; a.E = args->E; a.Tg = args->Tg;
   a.diag = args->diag; a.seasonal = args->seasonal; a.raw = args->raw; a.flags = args->flags;
   a.orig = (const long long*)args->member_index;
@@ -319,7 +497,6 @@ extern "C" int32_t ebm_classic_run_device(const ebm_grid_t* grid, const ebm_clas
     long long bits; memcpy(&bits, &ethr, sizeof(bits));
     a.hthr = (int)(bits >> 32);
   }
-  const int ypl = opt.years_per_launch > 0 ? opt.years_per_launch : grid->dur;
   // ---- launch-uniform parameters (a forcing sweep such as C4: members differ in forcing and initial state only).  The
   // member constants then travel in the kernel argument block and are constant-bank operands of the FP64 instructions;
   // the 26 registers they otherwise occupy go to instruction-level parallelism (classic_uniform.cu, UPAR).  The host
@@ -357,7 +534,7 @@ extern "C" int32_t ebm_classic_run_device(const ebm_grid_t* grid, const ebm_clas
     if (slots > 0 && blocks > slots && blocks <= 12 * slots && grid->dur >= 8 &&
         (double)(waves * slots) > 1.08 * (double)blocks) {
       constexpr int S = 8, nchunk = 16;   // measured flat between 4 x 20 and 16 x 40 (DESIGN.md)
-      const int chunk = std::min(ypl, std::max(1, grid->dur / nchunk));
+      const int chunk = std::min(opt.years_per_launch > 0 ? opt.years_per_launch : grid->dur, std::max(1, grid->dur / nchunk));
       cudaEvent_t fork;
       EBM_CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
       EBM_CUDA_TRY(cudaEventRecord(fork, stream));
@@ -391,12 +568,7 @@ extern "C" int32_t ebm_classic_run_device(const ebm_grid_t* grid, const ebm_clas
       return rc;
     }
   }
-  for (int y0 = 0; y0 < grid->dur; y0 += ypl) {
-    a.year0 = y0;
-    a.nyears = (y0 + ypl <= grid->dur) ? ypl : grid->dur - y0;
-    EBM_TRY(launch_classic(a, opt.strict != 0, stream));
-  }
-  return EBM_OK;
+  return launch_years(a, grid, opt, [&](const ClassicKArgs& b) { return launch_classic(b, opt.strict != 0, stream); });
 }
 
 extern "C" int32_t ebm_classic_run(const ebm_grid_t* grid, int64_t nmem, const ebm_classic_params_t* par,
@@ -404,105 +576,7 @@ extern "C" int32_t ebm_classic_run(const ebm_grid_t* grid, int64_t nmem, const e
                                    const ebm_options_t* opt_in, ebm_classic_outputs_t* out) {
   EBM_TRY(check_grid(grid));
   if (nmem < 1 || !par || !forc || !E0 || !Tg0 || !out) { ebm_set_error("classic_run: nmem >= 1 and par, forc, E0, Tg0, out must be non-NULL"); return EBM_ERR_INVALID; }
-  ebm_options_t opt = opt_in ? *opt_in : default_options();
-  DeviceRestore _dr;
-  EBM_TRY(select_device(opt));
-  if ((out->seasonal || out->raw) && opt.field_stride <= 0) { ebm_set_error("seasonal/raw output requested but field_stride == 0"); return EBM_ERR_INVALID; }
-  const int nx = grid->nx, nt = grid->nt, dur = grid->dur;
-  const long long nsel = nsel_of(nmem, opt.field_stride);
-  const long long nraw = opt.lastonly ? nt : (long long)nt * dur;
-  cudaStream_t s;
-  EBM_CUDA_TRY(cudaStreamCreate(&s));
-  DevBufs B;                 // declared first: destroyed last
-  StreamGuard sg{s};         // ... after the stream has drained (error paths return without a synchronise of their own)
-  double *stage, *dpar, *dforc, *dE, *dTg, *ddiag = nullptr, *dseas = nullptr, *draw = nullptr;
-  int* dflags = nullptr;
-  const size_t stage_n = (size_t)nmem * (nx > EBM_CLASSIC_NPAR ? nx : EBM_CLASSIC_NPAR);
-  EBM_TRY(B.alloc(&stage, stage_n));
-  EBM_TRY(B.alloc(&dpar, (size_t)nmem * EBM_CLASSIC_NPAR));
-  EBM_TRY(B.alloc(&dforc, (size_t)nmem * EBM_NFORCING));
-  EBM_TRY(B.alloc(&dE, (size_t)nmem * nx));
-  EBM_TRY(B.alloc(&dTg, (size_t)nmem * nx));
-  // Lanes of a warp are members: members in different regimes (snowball next to ice free) make every warp take
-  // both code paths.  Sort the members by the regime of their initial state (stable: the caller's order survives
-  // within a regime); the kernels write every output row at the member's original index (member_index).
-  std::vector<long long> perm;
-  long long* dperm = nullptr;
-  if (!opt.strict && nmem > 32) {
-    // primary key: the set of table-building parameters (D, S0, S2, a0, a2, cg, tau -- the table-driven kernel needs
-    // them uniform over 32-member groups), numbered in order of first appearance; secondary: regime of the initial
-    // state (0 ice free, 1 partial cover, 2 every cell ice).  Ensembles made of many distinct parameter sets
-    // (a pure sweep over D) are left in the caller's order within each regime.
-    std::map<std::array<double, kClassicNTablePar>, int> sets;
-    std::vector<int> key((size_t)nmem);
-    const double* prow = (const double*)par;
-    bool many_sets = false;
-    for (long long m = 0; m < nmem; ++m) {
-      int ice = 0;
-      for (int j = 0; j < nx; ++j) ice += E0[m * nx + j] < 0.0;
-      const int regime = ice == 0 ? 0 : (ice == nx ? 2 : 1);
-      int sid = 0;
-      if (!many_sets) {
-        std::array<double, kClassicNTablePar> tp;
-        for (int q = 0; q < kClassicNTablePar; ++q) tp[q] = prow[m * EBM_CLASSIC_NPAR + ebm_classic_table_par(q)];
-        auto it = sets.find(tp);
-        if (it == sets.end()) it = sets.emplace(tp, (int)sets.size()).first;
-        sid = it->second;
-        if ((long long)sets.size() * 32 > nmem) many_sets = true;   // groups cannot be made uniform anyway
-      }
-      key[m] = sid * 4 + regime;
-    }
-    if (many_sets) for (long long m = 0; m < nmem; ++m) key[m] &= 3;
-    bool sorted = true;
-    for (long long m = 1; m < nmem; ++m) if (key[m] < key[m - 1]) { sorted = false; break; }
-    if (!sorted) {
-      perm.resize((size_t)nmem);
-      for (long long m = 0; m < nmem; ++m) perm[m] = m;
-      std::stable_sort(perm.begin(), perm.end(), [&](long long a, long long b) { return key[a] < key[b]; });   // perm[slot] = original index
-      EBM_TRY(B.alloc(&dperm, (size_t)nmem));
-      EBM_CUDA_TRY(cudaMemcpyAsync(dperm, perm.data(), sizeof(long long) * nmem, cudaMemcpyHostToDevice, s));
-    }
-  }
-  auto upload = [&](const double* host, double* dst, long long cols) -> int {
-    if (!dperm) return upload_transposed(host, stage, dst, nmem, cols, s);
-    EBM_CUDA_TRY(cudaMemcpyAsync(stage, host, sizeof(double) * nmem * cols, cudaMemcpyHostToDevice, s));
-    return ebm_launch_gather_transpose(stage, dst, nmem, cols, dperm, 0, s);
-  };
-  auto download = [&](double* host, const double* src) -> int {      // device [nx][slots] -> host [nmem][nx], original order
-    if (!dperm) return download_transposed(host, stage, src, nx, nmem, s);
-    EBM_TRY(ebm_launch_gather_transpose(src, stage, nmem, nx, dperm, 1, s));
-    EBM_CUDA_TRY(cudaMemcpyAsync(host, stage, sizeof(double) * nmem * nx, cudaMemcpyDeviceToHost, s));
-    return EBM_OK;
-  };
-  EBM_TRY(upload((const double*)par, dpar, EBM_CLASSIC_NPAR));
-  EBM_TRY(upload((const double*)forc, dforc, EBM_NFORCING));
-  EBM_TRY(upload(E0, dE, nx));
-  EBM_TRY(upload(Tg0, dTg, nx));
-  const double kNaN = NAN;
-  const size_t ndiag = (size_t)nmem * dur * EBM_NSEASON * EBM_NDIAG;
-  const size_t nseas = (size_t)nsel * dur * EBM_NSEASON * EBM_CLASSIC_NVAR * nx;
-  const size_t nrawn = (size_t)nsel * nraw * EBM_CLASSIC_NVAR * nx;
-  if (out->diag) { EBM_TRY(B.alloc(&ddiag, ndiag)); EBM_TRY(ebm_launch_fill(ddiag, (long long)ndiag, kNaN, s)); }
-  if (out->seasonal) { EBM_TRY(B.alloc(&dseas, nseas)); EBM_TRY(ebm_launch_fill(dseas, (long long)nseas, kNaN, s)); }
-  if (out->raw) { EBM_TRY(B.alloc(&draw, nrawn)); EBM_TRY(ebm_launch_fill(draw, (long long)nrawn, kNaN, s)); }
-  if (out->flags) { EBM_TRY(B.alloc(&dflags, (size_t)nmem)); EBM_CUDA_TRY(cudaMemsetAsync(dflags, 0, sizeof(int) * nmem, s)); }
-  ebm_classic_device_args_t da;
-  memset(&da, 0, sizeof(da));
-  da.nmem = nmem; da.par = dpar; da.forc = dforc; da.E = dE; da.Tg = dTg;
-  da.diag = ddiag; da.seasonal = dseas; da.raw = draw; da.flags = dflags;
-  da.member_index = (const int64_t*)dperm;
-  EBM_TRY(ebm_classic_run_device(grid, &da, &opt, s));
-  if (out->diag) {
-    if (ebm_tl_diag_hook) EBM_TRY(ebm_tl_diag_hook->consume(ddiag, ndiag, s));
-    else EBM_CUDA_TRY(cudaMemcpyAsync(out->diag, ddiag, sizeof(double) * ndiag, cudaMemcpyDeviceToHost, s));
-  }
-  if (out->seasonal) EBM_CUDA_TRY(cudaMemcpyAsync(out->seasonal, dseas, sizeof(double) * nseas, cudaMemcpyDeviceToHost, s));
-  if (out->raw) EBM_CUDA_TRY(cudaMemcpyAsync(out->raw, draw, sizeof(double) * nrawn, cudaMemcpyDeviceToHost, s));
-  if (out->flags) EBM_CUDA_TRY(cudaMemcpyAsync(out->flags, dflags, sizeof(int) * nmem, cudaMemcpyDeviceToHost, s));
-  if (out->E_final) { EBM_TRY(download(out->E_final, dE)); EBM_CUDA_TRY(cudaStreamSynchronize(s)); }
-  if (out->Tg_final) { EBM_TRY(download(out->Tg_final, dTg)); }
-  EBM_CUDA_TRY(cudaStreamSynchronize(s));
-  return EBM_OK;
+  return ebm_run_host(grid, nmem, ebm_classic_host_run(par, forc, E0, Tg0, out), opt_in, nullptr);
 }
 
 extern "C" int32_t ebm_classic_step_debug(const ebm_grid_t* grid, const ebm_classic_params_t* par, int32_t ti, double f,
@@ -550,32 +624,18 @@ extern "C" int32_t ebm_miz_run_device(const ebm_grid_t* grid, const ebm_miz_devi
     ebm_set_error("miz_run_device: par, forc and the six state arrays must be non-NULL");
     return EBM_ERR_INVALID;
   }
-  if (args->nmem < 1) { ebm_set_error("nmem must be >= 1"); return EBM_ERR_INVALID; }
-  ebm_options_t opt = opt_in ? *opt_in : default_options();
+  const ebm_options_t opt = opt_in ? *opt_in : default_options();
   DeviceRestore _dr;
-  EBM_TRY(select_device(opt));
-  if ((args->seasonal || args->raw) && opt.field_stride <= 0) { ebm_set_error("seasonal/raw output requested but field_stride == 0"); return EBM_ERR_INVALID; }
   MizKArgs a;
-  memset(&a, 0, sizeof(a));
-  EBM_TRY(get_tables(grid, &a.g, stream));
-  a.nx = grid->nx; a.nt = grid->nt; a.dur = grid->dur; a.nmem = args->nmem;
-  a.winter_inx = grid->winter_inx; a.summer_inx = grid->summer_inx;
-  a.lastonly = opt.lastonly; a.field_stride = opt.field_stride;
+  EBM_TRY(device_prologue(grid, args, opt, &a, stream));
   a.maxit = opt.newton_maxit > 0 ? opt.newton_maxit : 100;
   a.tol = opt.newton_tol > 0.0 ? opt.newton_tol : 1e-8;
   a.step_limit = opt.step_limit > 0 ? opt.step_limit : 0;
-  a.start_year = opt.start_year > 0 ? opt.start_year : 0;
   a.par = args->par; a.forc = args->forc;
   a.Ei = args->Ei; a.Ew = args->Ew; a.h = args->h; a.D = args->D; a.phi = args->phi; a.T0 = args->T0;
   a.diag = args->diag; a.seasonal = args->seasonal; a.raw = args->raw;
   a.newton_iters = (long long*)args->newton_iters; a.nonconv = (long long*)args->nonconv; a.flags = args->flags;
-  const int ypl = opt.years_per_launch > 0 ? opt.years_per_launch : grid->dur;
-  for (int y0 = 0; y0 < grid->dur; y0 += ypl) {
-    a.year0 = y0;
-    a.nyears = (y0 + ypl <= grid->dur) ? ypl : grid->dur - y0;
-    EBM_TRY(ebm_launch_miz(a, opt.strict, stream));
-  }
-  return EBM_OK;
+  return launch_years(a, grid, opt, [&](const MizKArgs& b) { return ebm_launch_miz(b, opt.strict, stream); });
 }
 
 extern "C" int32_t ebm_miz_run(const ebm_grid_t* grid, int64_t nmem, const ebm_miz_params_t* par,
@@ -584,63 +644,7 @@ extern "C" int32_t ebm_miz_run(const ebm_grid_t* grid, int64_t nmem, const ebm_m
                                const ebm_options_t* opt_in, ebm_miz_outputs_t* out) {
   EBM_TRY(check_grid(grid));
   if (nmem < 1 || !par || !forc || !Ei0 || !Ew0 || !h0 || !D0 || !phi0 || !out) { ebm_set_error("miz_run: NULL argument or nmem < 1"); return EBM_ERR_INVALID; }
-  ebm_options_t opt = opt_in ? *opt_in : default_options();
-  DeviceRestore _dr;
-  EBM_TRY(select_device(opt));
-  if ((out->seasonal || out->raw) && opt.field_stride <= 0) { ebm_set_error("seasonal/raw output requested but field_stride == 0"); return EBM_ERR_INVALID; }
-  const int nx = grid->nx, nt = grid->nt, dur = grid->dur;
-  const long long nsel = nsel_of(nmem, opt.field_stride);
-  const long long nraw = opt.lastonly ? nt : (long long)nt * dur;
-  cudaStream_t s;
-  EBM_CUDA_TRY(cudaStreamCreate(&s));
-  DevBufs B;                 // declared first: destroyed last
-  StreamGuard sg{s};         // ... after the stream has drained (error paths return without a synchronise of their own)
-  double *stage, *dpar, *dforc, *dst[6], *ddiag = nullptr, *dseas = nullptr, *draw = nullptr;
-  long long *dit = nullptr, *dnc = nullptr;
-  int* dflags = nullptr;
-  const size_t stage_n = (size_t)nmem * (nx > EBM_MIZ_NPAR ? nx : EBM_MIZ_NPAR);
-  EBM_TRY(B.alloc(&stage, stage_n));
-  EBM_TRY(B.alloc(&dpar, (size_t)nmem * EBM_MIZ_NPAR));
-  EBM_TRY(B.alloc(&dforc, (size_t)nmem * EBM_NFORCING));
-  EBM_TRY(upload_transposed((const double*)par, stage, dpar, nmem, EBM_MIZ_NPAR, s));
-  EBM_TRY(upload_transposed((const double*)forc, stage, dforc, nmem, EBM_NFORCING, s));
-  const double* init[6] = {Ei0, Ew0, h0, D0, phi0, T0guess};
-  for (int q = 0; q < 6; ++q) {
-    EBM_TRY(B.alloc(&dst[q], (size_t)nmem * nx));
-    if (init[q]) EBM_TRY(upload_transposed(init[q], stage, dst[q], nmem, nx, s));
-    else EBM_CUDA_TRY(cudaMemsetAsync(dst[q], 0, sizeof(double) * nmem * nx, s));
-  }
-  const double kNaN = NAN;
-  const size_t ndiag = (size_t)nmem * dur * EBM_NSEASON * EBM_NDIAG;
-  const size_t nseas = (size_t)nsel * dur * EBM_NSEASON * EBM_MIZ_NVAR * nx;
-  const size_t nrawn = (size_t)nsel * nraw * EBM_MIZ_NVAR * nx;
-  if (out->diag) { EBM_TRY(B.alloc(&ddiag, ndiag)); EBM_TRY(ebm_launch_fill(ddiag, (long long)ndiag, kNaN, s)); }
-  if (out->seasonal) { EBM_TRY(B.alloc(&dseas, nseas)); EBM_TRY(ebm_launch_fill(dseas, (long long)nseas, kNaN, s)); }
-  if (out->raw) { EBM_TRY(B.alloc(&draw, nrawn)); EBM_TRY(ebm_launch_fill(draw, (long long)nrawn, kNaN, s)); }
-  EBM_TRY(B.alloc(&dit, (size_t)nmem)); EBM_CUDA_TRY(cudaMemsetAsync(dit, 0, sizeof(long long) * nmem, s));
-  EBM_TRY(B.alloc(&dnc, (size_t)nmem)); EBM_CUDA_TRY(cudaMemsetAsync(dnc, 0, sizeof(long long) * nmem, s));
-  EBM_TRY(B.alloc(&dflags, (size_t)nmem)); EBM_CUDA_TRY(cudaMemsetAsync(dflags, 0, sizeof(int) * nmem, s));
-  ebm_miz_device_args_t da;
-  memset(&da, 0, sizeof(da));
-  da.nmem = nmem; da.par = dpar; da.forc = dforc;
-  da.Ei = dst[0]; da.Ew = dst[1]; da.h = dst[2]; da.D = dst[3]; da.phi = dst[4]; da.T0 = dst[5];
-  da.diag = ddiag; da.seasonal = dseas; da.raw = draw;
-  da.newton_iters = (int64_t*)dit; da.nonconv = (int64_t*)dnc; da.flags = dflags;
-  EBM_TRY(ebm_miz_run_device(grid, &da, &opt, s));
-  if (out->diag) {
-    if (ebm_tl_diag_hook) EBM_TRY(ebm_tl_diag_hook->consume(ddiag, ndiag, s));
-    else EBM_CUDA_TRY(cudaMemcpyAsync(out->diag, ddiag, sizeof(double) * ndiag, cudaMemcpyDeviceToHost, s));
-  }
-  if (out->seasonal) EBM_CUDA_TRY(cudaMemcpyAsync(out->seasonal, dseas, sizeof(double) * nseas, cudaMemcpyDeviceToHost, s));
-  if (out->raw) EBM_CUDA_TRY(cudaMemcpyAsync(out->raw, draw, sizeof(double) * nrawn, cudaMemcpyDeviceToHost, s));
-  if (out->newton_iters) EBM_CUDA_TRY(cudaMemcpyAsync(out->newton_iters, dit, sizeof(long long) * nmem, cudaMemcpyDeviceToHost, s));
-  if (out->nonconv) EBM_CUDA_TRY(cudaMemcpyAsync(out->nonconv, dnc, sizeof(long long) * nmem, cudaMemcpyDeviceToHost, s));
-  if (out->flags) EBM_CUDA_TRY(cudaMemcpyAsync(out->flags, dflags, sizeof(int) * nmem, cudaMemcpyDeviceToHost, s));
-  double* fin[6] = {out->Ei_final, out->Ew_final, out->h_final, out->D_final, out->phi_final, out->T0_final};
-  for (int q = 0; q < 6; ++q)
-    if (fin[q]) { EBM_TRY(download_transposed(fin[q], stage, dst[q], nx, nmem, s)); EBM_CUDA_TRY(cudaStreamSynchronize(s)); }
-  EBM_CUDA_TRY(cudaStreamSynchronize(s));
-  return EBM_OK;
+  return ebm_run_host(grid, nmem, ebm_miz_host_run(par, forc, Ei0, Ew0, h0, D0, phi0, T0guess, out), opt_in, nullptr);
 }
 
 extern "C" int32_t ebm_miz_step(const ebm_grid_t* grid, const ebm_miz_params_t* par, int32_t ti, double f,

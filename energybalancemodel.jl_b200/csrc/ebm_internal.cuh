@@ -4,6 +4,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <vector>
+
 #include "ebm_cuda.h"
 
 // ----------------------------------------------------------------------------- error plumbing
@@ -18,15 +20,44 @@ void ebm_count_launch(int n = 1);
       return (_e == cudaErrorMemoryAllocation) ? EBM_ERR_OOM : EBM_ERR_CUDA;                      \
     }                                                                                             \
   } while (0)
+#define EBM_TRY(expr) do { int _rc = (expr); if (_rc != EBM_OK) return _rc; } while (0)
 
-// ----------------------------------------------------------------------------- multi-device hook (ebm_multi.cu)
-// While set (thread local), the host entry points hand the device-resident diagnostics of their run to the hook
-// instead of copying them to out->diag: ebm_*_run_multi uses it to send them to another GPU over NCCL.
+// ----------------------------------------------------------------------------- host-buffer runs (ebm_capi.cu)
+// One call of ebm_classic_run or ebm_miz_run, described by the arrays its model carries.  Host arrays are
+// [nmem][...]; an output pointer may be NULL (not wanted).
+struct EbmHostRun {
+  int npar, nvar, nstate;                 // nstate: classic 2 (E, Tg); MIZ 6 (Ei, Ew, h, D, phi, T0)
+  const double* par; const double* forc;  // [nmem][npar], [nmem][EBM_NFORCING]
+  const double* init[6];                  // [nmem][nx]; NULL uploads zeros (MIZ T0guess only)
+  double* diag; double* seasonal; double* raw;
+  double* fin[6];                         // final state planes
+  int64_t* newton_iters; int64_t* nonconv; int32_t* flags;
+  // The model's device entry point, called with a copy of this description whose arrays are on the device ([...][nmem];
+  // the state planes, updated in place, are `fin`).  member_index: NULL or the permutation `order` returned.
+  int (*run_device)(const ebm_grid_t* grid, long long nmem, const EbmHostRun& dev, const long long* member_index,
+                    const ebm_options_t& opt, cudaStream_t stream);
+  // NULL, or the order in which the members go to the device: perm[slot] = original index; empty = the caller's order
+  std::vector<long long> (*order)(const ebm_grid_t* grid, long long nmem, const EbmHostRun& run, const ebm_options_t& opt);
+};
+EbmHostRun ebm_classic_host_run(const ebm_classic_params_t* par, const ebm_forcing_t* forc, const double* E0,
+                                const double* Tg0, const ebm_classic_outputs_t* out);
+EbmHostRun ebm_miz_host_run(const ebm_miz_params_t* par, const ebm_forcing_t* forc, const double* Ei0, const double* Ew0,
+                            const double* h0, const double* D0, const double* phi0, const double* T0guess,
+                            const ebm_miz_outputs_t* out);
+// Receives the device-resident diagnostics of a host run instead of a copy to run.diag: ebm_*_run_multi sends them
+// to another GPU over NCCL.
 struct EbmDiagHook {
   virtual int consume(const double* ddiag, size_t count, cudaStream_t stream) = 0;   // EBM_* status
   virtual ~EbmDiagHook() {}
 };
-extern thread_local EbmDiagHook* ebm_tl_diag_hook;
+// Uploads, integrates on a private stream of opt->device and downloads; diag_hook (may be NULL) takes the diagnostics.
+int ebm_run_host(const ebm_grid_t* grid, long long nmem, const EbmHostRun& run, const ebm_options_t* opt,
+                 EbmDiagHook* diag_hook);
+ebm_options_t default_options();   // device -1, lastonly 1, everything else 0
+// Classic regime of one member's state E [nx]: 0 ice free, 1 partial cover, 2 every cell ice.
+int ebm_classic_regime(const double* E, int nx);
+
+// ----------------------------------------------------------------------------- multi-device (ebm_multi.cu)
 int ebm_launch_scatter_rows(const double* src, double* dst, long long nrows, long long rowlen, const long long* idx,
                             cudaStream_t stream);   // dst[idx[r]][:] = src[r][:]
 void ebm_multi_shutdown();   // destroys the NCCL communicators of ebm_multi.cu

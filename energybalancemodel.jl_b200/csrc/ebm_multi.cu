@@ -6,15 +6,15 @@
 //   * members are dealt to the GPUs in packets of 32 after a stable sort by what they cost (classic: the regime of the
 //     initial state) -- a contiguous cut of an ensemble ordered by a physical parameter hands one GPU all the expensive
 //     members (round-1 VERDICT: the rank holding F = -20... set the step time);
-//   * every thread runs the ordinary host entry point (ebm_classic_run / ebm_miz_run) on its members and scatters the
+//   * every thread runs the host run of ebm_classic_run / ebm_miz_run (ebm_run_host) on its members and scatters the
 //     rows it gets back to the caller's arrays at the members' original indices;
 //   * diagnostics: with multi->diag_device < 0 every GPU copies its own rows to the caller's host buffer; with
 //     diag_device >= 0 the caller's `diag` is DEVICE memory on that GPU and the other GPUs send their rows there over
-//     NVLink: ncclSend / ncclRecv on communicators this library owns (ncclCommInitAll, created lazily per device set,
-//     destroyed by ebm_shutdown).  NCCL is bound with dlopen("libnccl.so.2") at first use, so the library has no
-//     link-time dependency on it and shares the copy a host process (e.g. torch) has already loaded.
-// Field outputs (seasonal / raw) are per-member opt-ins of single-GPU runs; the multi-GPU entry points return
-// EBM_ERR_UNSUPPORTED for them.
+//     NVLink: each thread passes its host run a GatherHook, which takes the device-resident rows and runs ncclSend /
+//     ncclRecv on communicators this library owns (ncclCommInitAll, created lazily per device set, destroyed by
+//     ebm_shutdown).  NCCL is bound with dlopen("libnccl.so.2") at first use, so the library has no link-time
+//     dependency on it and shares the copy a host process (e.g. torch) has already loaded;
+//   * field outputs (seasonal / raw): each GPU integrates its field-selected members once more (FieldSel).
 #include <dlfcn.h>
 #include <nccl.h>
 #include <string.h>
@@ -188,13 +188,13 @@ struct GatherHook : EbmDiagHook {
 // neighbours, so the fields belong bit for bit to the run that produced the diagnostics -- and their rows land at
 // global index / field_stride in the caller's arrays.
 struct FieldSel {
-  std::vector<long long> local, slot;   // position in the device's sub-ensemble, row in the caller's field arrays
+  std::vector<long long> member, slot;   // the member's index, its row in the caller's field arrays
   FieldSel(const std::vector<long long>& ix, int stride, bool wanted) {
     if (!wanted || stride <= 0) return;
-    for (size_t r = 0; r < ix.size(); ++r)
-      if (ix[r] % stride == 0) { local.push_back((long long)r); slot.push_back(ix[r] / stride); }
+    for (long long m : ix)
+      if (m % stride == 0) { member.push_back(m); slot.push_back(m / stride); }
   }
-  bool any() const { return !local.empty(); }
+  bool any() const { return !member.empty(); }
 };
 
 struct ThreadResult { int rc = EBM_OK; std::string err; };
@@ -237,24 +237,38 @@ void ebm_multi_shutdown() {
   g_comms.clear();
 }
 
-extern "C" int32_t ebm_classic_run_multi(const ebm_grid_t* grid, int64_t nmem, const ebm_classic_params_t* par,
-                                         const ebm_forcing_t* forc, const double* E0, const double* Tg0,
-                                         const ebm_options_t* opt_in, const ebm_multi_t* multi, ebm_classic_outputs_t* out) {
-  if (!grid || nmem < 1 || !par || !forc || !E0 || !Tg0 || !out) { ebm_set_error("classic_run_multi: NULL argument or nmem < 1"); return EBM_ERR_INVALID; }
+namespace {
+
+// The members `ix` of `run`: their input rows, copied into `rows`, and no output wanted.
+struct MemberRows { std::vector<double> par, forc, init[6]; };
+EbmHostRun members(const EbmHostRun& run, const std::vector<long long>& ix, int nx, MemberRows* rows) {
+  EbmHostRun r = run;
+  rows->par = take_rows(run.par, ix, (size_t)run.npar);
+  rows->forc = take_rows(run.forc, ix, EBM_NFORCING);
+  r.par = rows->par.data(); r.forc = rows->forc.data();
+  for (int k = 0; k < run.nstate; ++k) {
+    if (run.init[k]) rows->init[k] = take_rows(run.init[k], ix, (size_t)nx);
+    r.init[k] = run.init[k] ? rows->init[k].data() : nullptr;
+    r.fin[k] = nullptr;
+  }
+  r.diag = r.seasonal = r.raw = nullptr;
+  r.newton_iters = r.nonconv = nullptr;
+  r.flags = nullptr;
+  return r;
+}
+
+// The per-device body of both models: every thread runs the host run of its members, puts their rows back at the
+// members' original indices and reruns its field-selected members with field_stride = 1.  key: deal key (may be empty).
+int run_multi(const ebm_grid_t* grid, long long nmem, const EbmHostRun& run, const std::vector<int>& key,
+              const ebm_options_t* opt_in, const ebm_multi_t* multi) {
   std::vector<int> devs;
   int rc = resolve_devices(multi, &devs);
   if (rc != EBM_OK) return rc;
   const int ndev = (int)devs.size(), nx = grid->nx;
   const size_t rowlen = (size_t)grid->dur * EBM_NSEASON * EBM_NDIAG;
-  std::vector<int> key((size_t)nmem);
-  for (long long m = 0; m < nmem; ++m) {
-    int ice = 0;
-    for (int j = 0; j < nx; ++j) ice += E0[m * nx + j] < 0.0;
-    key[(size_t)m] = ice == 0 ? 0 : (ice == nx ? 2 : 1);
-  }
   NcclGather g;
   g.idx = deal(nmem, ndev, key, (multi && multi->packet > 0) ? multi->packet : 32);
-  const int nccl = setup_gather(multi, devs, &g, out->diag, rowlen);
+  const int nccl = setup_gather(multi, devs, &g, run.diag, rowlen);
   if (nccl < 0) return nccl;
   return run_threads(ndev, [&](int q) -> int {
     const auto& ix = g.idx[(size_t)q];
@@ -267,51 +281,55 @@ extern "C" int32_t ebm_classic_run_multi(const ebm_grid_t* grid, int64_t nmem, c
       EBM_CUDA_TRY(cudaStreamSynchronize(0));
       return r0;
     }
-    auto p = take_rows((const double*)par, ix, EBM_CLASSIC_NPAR);
-    auto f = take_rows((const double*)forc, ix, EBM_NFORCING);
-    auto e = take_rows(E0, ix, (size_t)nx), t = take_rows(Tg0, ix, (size_t)nx);
-    std::vector<double> dg(out->diag && !nccl ? n * rowlen : 0), ef(out->E_final ? n * nx : 0), tf(out->Tg_final ? n * nx : 0);
-    std::vector<int32_t> fl(out->flags ? n : 0);
-    ebm_classic_outputs_t o;
-    memset(&o, 0, sizeof(o));
-    o.diag = out->diag ? (nccl ? out->diag /* marker: wanted; the hook takes the rows */ : dg.data()) : nullptr;
-    o.E_final = out->E_final ? ef.data() : nullptr;
-    o.Tg_final = out->Tg_final ? tf.data() : nullptr;
-    o.flags = out->flags ? fl.data() : nullptr;
-    ebm_options_t op;
-    if (opt_in) op = *opt_in; else { memset(&op, 0, sizeof(op)); op.lastonly = 1; }
+    MemberRows in;
+    EbmHostRun r = members(run, ix, nx, &in);
+    std::vector<double> fin[6], dg(run.diag && !nccl ? n * rowlen : 0);
+    for (int k = 0; k < run.nstate; ++k) {
+      if (run.fin[k]) fin[k].resize(n * nx);
+      r.fin[k] = run.fin[k] ? fin[k].data() : nullptr;
+    }
+    std::vector<int64_t> it(run.newton_iters ? n : 0), nc(run.nonconv ? n : 0);
+    std::vector<int32_t> fl(run.flags ? n : 0);
+    r.diag = run.diag && !nccl ? dg.data() : nullptr;
+    r.newton_iters = run.newton_iters ? it.data() : nullptr;
+    r.nonconv = run.nonconv ? nc.data() : nullptr;
+    r.flags = run.flags ? fl.data() : nullptr;
+    ebm_options_t op = opt_in ? *opt_in : default_options();
     op.device = devs[(size_t)q];
     op.field_stride = 0;
-    ebm_tl_diag_hook = nccl ? &hook : nullptr;
-    const int r = ebm_classic_run(grid, (int64_t)n, (const ebm_classic_params_t*)p.data(), (const ebm_forcing_t*)f.data(),
-                                  e.data(), t.data(), &op, &o);
-    ebm_tl_diag_hook = nullptr;
-    if (r != EBM_OK) return r;
-    if (!nccl) put_rows(out->diag, dg, ix, rowlen);
-    put_rows(out->E_final, ef, ix, (size_t)nx);
-    put_rows(out->Tg_final, tf, ix, (size_t)nx);
-    put_rows(out->flags, fl, ix, 1);
-    const FieldSel fs(ix, opt_in ? opt_in->field_stride : 0, out->seasonal || out->raw);
+    EBM_TRY(ebm_run_host(grid, (long long)n, r, &op, nccl ? &hook : nullptr));
+    if (!nccl) put_rows(run.diag, dg, ix, rowlen);
+    for (int k = 0; k < run.nstate; ++k) put_rows(run.fin[k], fin[k], ix, (size_t)nx);
+    put_rows(run.newton_iters, it, ix, 1);
+    put_rows(run.nonconv, nc, ix, 1);
+    put_rows(run.flags, fl, ix, 1);
+    const FieldSel fs(ix, opt_in ? opt_in->field_stride : 0, run.seasonal || run.raw);
     if (fs.any()) {
-      const size_t ns = fs.local.size(), nraw = (size_t)(op.lastonly ? grid->nt : (long long)grid->nt * grid->dur);
-      const size_t lenS = (size_t)grid->dur * EBM_NSEASON * EBM_CLASSIC_NVAR * nx, lenR = nraw * EBM_CLASSIC_NVAR * nx;
-      auto p2 = take_rows(p.data(), fs.local, EBM_CLASSIC_NPAR);
-      auto f2 = take_rows(f.data(), fs.local, EBM_NFORCING);
-      auto e2 = take_rows(e.data(), fs.local, (size_t)nx), t2 = take_rows(t.data(), fs.local, (size_t)nx);
-      std::vector<double> se(out->seasonal ? ns * lenS : 0), rw(out->raw ? ns * lenR : 0);
-      ebm_classic_outputs_t o2;
-      memset(&o2, 0, sizeof(o2));
-      o2.seasonal = out->seasonal ? se.data() : nullptr;
-      o2.raw = out->raw ? rw.data() : nullptr;
+      const size_t ns = fs.member.size(), nraw = (size_t)(op.lastonly ? grid->nt : (long long)grid->nt * grid->dur);
+      const size_t lenS = (size_t)grid->dur * EBM_NSEASON * run.nvar * nx, lenR = nraw * run.nvar * nx;
+      MemberRows in2;
+      EbmHostRun r2 = members(run, fs.member, nx, &in2);
+      std::vector<double> se(run.seasonal ? ns * lenS : 0), rw(run.raw ? ns * lenR : 0);
+      r2.seasonal = run.seasonal ? se.data() : nullptr;
+      r2.raw = run.raw ? rw.data() : nullptr;
       op.field_stride = 1;
-      const int r2 = ebm_classic_run(grid, (int64_t)ns, (const ebm_classic_params_t*)p2.data(), (const ebm_forcing_t*)f2.data(),
-                                     e2.data(), t2.data(), &op, &o2);
-      if (r2 != EBM_OK) return r2;
-      put_rows(out->seasonal, se, fs.slot, lenS);
-      put_rows(out->raw, rw, fs.slot, lenR);
+      EBM_TRY(ebm_run_host(grid, (long long)ns, r2, &op, nullptr));
+      put_rows(run.seasonal, se, fs.slot, lenS);
+      put_rows(run.raw, rw, fs.slot, lenR);
     }
     return EBM_OK;
   });
+}
+
+}  // namespace
+
+extern "C" int32_t ebm_classic_run_multi(const ebm_grid_t* grid, int64_t nmem, const ebm_classic_params_t* par,
+                                         const ebm_forcing_t* forc, const double* E0, const double* Tg0,
+                                         const ebm_options_t* opt_in, const ebm_multi_t* multi, ebm_classic_outputs_t* out) {
+  if (!grid || nmem < 1 || !par || !forc || !E0 || !Tg0 || !out) { ebm_set_error("classic_run_multi: NULL argument or nmem < 1"); return EBM_ERR_INVALID; }
+  std::vector<int> key((size_t)nmem);
+  for (long long m = 0; m < nmem; ++m) key[(size_t)m] = ebm_classic_regime(E0 + m * grid->nx, grid->nx);
+  return run_multi(grid, nmem, ebm_classic_host_run(par, forc, E0, Tg0, out), key, opt_in, multi);
 }
 
 extern "C" int32_t ebm_miz_run_multi(const ebm_grid_t* grid, int64_t nmem, const ebm_miz_params_t* par,
@@ -319,80 +337,6 @@ extern "C" int32_t ebm_miz_run_multi(const ebm_grid_t* grid, int64_t nmem, const
                                      const double* D0, const double* phi0, const double* T0guess,
                                      const ebm_options_t* opt_in, const ebm_multi_t* multi, ebm_miz_outputs_t* out) {
   if (!grid || nmem < 1 || !par || !forc || !Ei0 || !Ew0 || !h0 || !D0 || !phi0 || !out) { ebm_set_error("miz_run_multi: NULL argument or nmem < 1"); return EBM_ERR_INVALID; }
-  std::vector<int> devs;
-  int rc = resolve_devices(multi, &devs);
-  if (rc != EBM_OK) return rc;
-  const int ndev = (int)devs.size(), nx = grid->nx;
-  const size_t rowlen = (size_t)grid->dur * EBM_NSEASON * EBM_NDIAG;
-  NcclGather g;
-  g.idx = deal(nmem, ndev, std::vector<int>(), (multi && multi->packet > 0) ? multi->packet : 32);
-  const int nccl = setup_gather(multi, devs, &g, out->diag, rowlen);
-  if (nccl < 0) return nccl;
-  return run_threads(ndev, [&](int q) -> int {
-    const auto& ix = g.idx[(size_t)q];
-    const size_t n = ix.size();
-    GatherHook hook(&g, q);
-    if (n == 0) {   // no member for this GPU (fewer packets than devices): it still takes part in the exchange
-      if (!nccl) return EBM_OK;
-      EBM_CUDA_TRY(cudaSetDevice(devs[(size_t)q]));
-      const int r0 = hook.consume(nullptr, 0, 0);
-      EBM_CUDA_TRY(cudaStreamSynchronize(0));
-      return r0;
-    }
-    auto p = take_rows((const double*)par, ix, EBM_MIZ_NPAR);
-    auto f = take_rows((const double*)forc, ix, EBM_NFORCING);
-    const double* init[6] = {Ei0, Ew0, h0, D0, phi0, T0guess};
-    std::vector<double> in[6];
-    for (int k = 0; k < 6; ++k) if (init[k]) in[k] = take_rows(init[k], ix, (size_t)nx);
-    double* fin_dst[6] = {out->Ei_final, out->Ew_final, out->h_final, out->D_final, out->phi_final, out->T0_final};
-    std::vector<double> fin[6];
-    for (int k = 0; k < 6; ++k) if (fin_dst[k]) fin[k].resize(n * nx);
-    std::vector<double> dg(out->diag && !nccl ? n * rowlen : 0);
-    std::vector<int64_t> it(out->newton_iters ? n : 0), nc(out->nonconv ? n : 0);
-    std::vector<int32_t> fl(out->flags ? n : 0);
-    ebm_miz_outputs_t o;
-    memset(&o, 0, sizeof(o));
-    o.diag = out->diag ? (nccl ? out->diag : dg.data()) : nullptr;
-    o.Ei_final = fin_dst[0] ? fin[0].data() : nullptr; o.Ew_final = fin_dst[1] ? fin[1].data() : nullptr;
-    o.h_final = fin_dst[2] ? fin[2].data() : nullptr; o.D_final = fin_dst[3] ? fin[3].data() : nullptr;
-    o.phi_final = fin_dst[4] ? fin[4].data() : nullptr; o.T0_final = fin_dst[5] ? fin[5].data() : nullptr;
-    o.newton_iters = out->newton_iters ? it.data() : nullptr;
-    o.nonconv = out->nonconv ? nc.data() : nullptr;
-    o.flags = out->flags ? fl.data() : nullptr;
-    ebm_options_t op;
-    if (opt_in) op = *opt_in; else { memset(&op, 0, sizeof(op)); op.lastonly = 1; }
-    op.device = devs[(size_t)q];
-    op.field_stride = 0;
-    ebm_tl_diag_hook = nccl ? &hook : nullptr;
-    const int r = ebm_miz_run(grid, (int64_t)n, (const ebm_miz_params_t*)p.data(), (const ebm_forcing_t*)f.data(), in[0].data(),
-                              in[1].data(), in[2].data(), in[3].data(), in[4].data(), init[5] ? in[5].data() : nullptr, &op, &o);
-    ebm_tl_diag_hook = nullptr;
-    if (r != EBM_OK) return r;
-    if (!nccl) put_rows(out->diag, dg, ix, rowlen);
-    for (int k = 0; k < 6; ++k) put_rows(fin_dst[k], fin[k], ix, (size_t)nx);
-    put_rows(out->newton_iters, it, ix, 1);
-    put_rows(out->nonconv, nc, ix, 1);
-    put_rows(out->flags, fl, ix, 1);
-    const FieldSel fs(ix, opt_in ? opt_in->field_stride : 0, out->seasonal || out->raw);
-    if (fs.any()) {
-      const size_t ns = fs.local.size(), nraw = (size_t)(op.lastonly ? grid->nt : (long long)grid->nt * grid->dur);
-      const size_t lenS = (size_t)grid->dur * EBM_NSEASON * EBM_MIZ_NVAR * nx, lenR = nraw * EBM_MIZ_NVAR * nx;
-      auto p2 = take_rows(p.data(), fs.local, EBM_MIZ_NPAR);
-      auto f2 = take_rows(f.data(), fs.local, EBM_NFORCING);
-      std::vector<double> in2[6];
-      for (int k = 0; k < 6; ++k) if (init[k]) in2[k] = take_rows(in[k].data(), fs.local, (size_t)nx);
-      std::vector<double> se(out->seasonal ? ns * lenS : 0), rw(out->raw ? ns * lenR : 0);
-      ebm_miz_outputs_t o2;
-      memset(&o2, 0, sizeof(o2));
-      o2.seasonal = out->seasonal ? se.data() : nullptr;
-      o2.raw = out->raw ? rw.data() : nullptr;
-      op.field_stride = 1;
-      const int r2 = ebm_miz_run(grid, (int64_t)ns, (const ebm_miz_params_t*)p2.data(), (const ebm_forcing_t*)f2.data(), in2[0].data(),
-                                 in2[1].data(), in2[2].data(), in2[3].data(), in2[4].data(), init[5] ? in2[5].data() : nullptr, &op, &o2);
-      if (r2 != EBM_OK) return r2;
-      put_rows(out->seasonal, se, fs.slot, lenS);
-      put_rows(out->raw, rw, fs.slot, lenR);
-    }
-    return EBM_OK;
-  });
+  return run_multi(grid, nmem, ebm_miz_host_run(par, forc, Ei0, Ew0, h0, D0, phi0, T0guess, out), std::vector<int>(), opt_in,
+                   multi);
 }

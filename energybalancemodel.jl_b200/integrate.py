@@ -8,6 +8,7 @@ numerical operation happens in libebm_cuda.so; there is no CPU fallback.
 from __future__ import annotations
 
 import ctypes as C
+from collections import namedtuple
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -20,7 +21,18 @@ __all__ = ["integrate", "integrate_ensemble", "integrate_arrays", "integrate_gri
            "fp64_peak", "model_name"]
 
 _MIZ_STATE = ("Ei", "Ew", "h", "D", "phi")
-_CLASSIC_STATE = ("E", "Tg")
+
+
+# What the host entry points of a model take and return (include/ebm_cuda.h): parameter order, stored variables, initial
+# state in argument order, whether the closure warm start T0 follows it (optional on input; always returned), the
+# int64 per-member counters, the outputs struct and the single- and multi-GPU entry points.
+_Model = namedtuple("_Model", "par_order variables state T0 counters outputs run run_multi")
+_MODELS = {
+    "Classic": _Model(CLASSIC_PAR_ORDER, CLASSIC_VARS, ("E", "Tg"), False, (), _lib.ClassicOutputs,
+                      "ebm_classic_run", "ebm_classic_run_multi"),
+    "MIZ": _Model(MIZ_PAR_ORDER, MIZ_VARS, _MIZ_STATE, True, ("newton_iters", "nonconv"), _lib.MizOutputs,
+                  "ebm_miz_run", "ebm_miz_run_multi"),
+}
 
 
 def model_name(model) -> str:
@@ -92,14 +104,11 @@ def integrate_ensemble(model, st: SpaceTime, forcings, pars, inits, *, T0guess=N
     if not (len(forcings) == nmem == len(inits)) or nmem == 0:
         raise ValueError("forcings, pars and inits must be non-empty and of equal length")
     forc = np.stack([f.row() for f in forcings])
-    if name == "Classic":
-        par = _rows(pars, CLASSIC_PAR_ORDER)
-        state = {k: _stack(inits, k, st.nx) for k in _CLASSIC_STATE}
-    else:
-        par = _rows(pars, MIZ_PAR_ORDER)
-        state = {k: _stack(inits, k, st.nx) for k in _MIZ_STATE}
-        if T0guess is not None:
-            state["T0"] = np.asarray(T0guess, dtype=np.float64).reshape(nmem, st.nx)
+    m = _MODELS[name]
+    par = _rows(pars, m.par_order)
+    state = {k: _stack(inits, k, st.nx) for k in m.state}
+    if m.T0 and T0guess is not None:
+        state["T0"] = np.asarray(T0guess, dtype=np.float64).reshape(nmem, st.nx)
     return integrate_arrays(name, st, forc, par, state, **kw)
 
 
@@ -169,9 +178,10 @@ def integrate_arrays(model, st: SpaceTime, forc, par, state, *, lastonly: bool =
     (src/infrastructure.jl:500-527) instead of ``get_diffop(nx)``, i.e. the classic model on non-uniform grids; the
     default 0 reproduces the reference, which uses ``get_diffop`` whatever the grid (src/classic.jl:21)."""
     name = model_name(model)
+    m = _MODELS[name]
     lib = _lib.load()
     nx, nt, dur = st.nx, st.nt, st.dur
-    npar = len(CLASSIC_PAR_ORDER) if name == "Classic" else len(MIZ_PAR_ORDER)
+    npar = len(m.par_order)
     par = np.ascontiguousarray(par, dtype=np.float64)
     forc = np.ascontiguousarray(forc, dtype=np.float64)
     if par.ndim != 2 or par.shape[1] != npar or par.shape[0] == 0:
@@ -179,9 +189,8 @@ def integrate_arrays(model, st: SpaceTime, forc, par, state, *, lastonly: bool =
     nmem = par.shape[0]
     if forc.shape != (nmem, _lib.NFORCING):
         raise ValueError(f"forc must be [nmem, {_lib.NFORCING}] (Forcing.row() layout)")
-    keys = _CLASSIC_STATE if name == "Classic" else _MIZ_STATE
     arrs = {}
-    for k in keys + (("T0",) if (name == "MIZ" and "T0" in state) else ()):
+    for k in m.state + (("T0",) if (m.T0 and "T0" in state) else ()):
         if k not in state:
             raise KeyError(f"initial state lacks {k!r}")
         a = np.ascontiguousarray(state[k], dtype=np.float64)
@@ -200,39 +209,24 @@ def integrate_arrays(model, st: SpaceTime, forc, par, state, *, lastonly: bool =
         want_seasonal = nsel > 0
     if want_raw is None:
         want_raw = nsel > 0
-    variables = CLASSIC_VARS if name == "Classic" else MIZ_VARS
-    nvar = len(variables)
-    res = EnsembleResult(name, st, nmem, field_stride, variables)
+    nvar = len(m.variables)
+    res = EnsembleResult(name, st, nmem, field_stride, m.variables)
     res.diag = np.empty((nmem, dur, 3, 4)) if want_diag else None
     res.seasonal = np.empty((nsel, dur, 3, nvar, nx)) if (want_seasonal and nsel) else None
     res.raw = np.empty((nsel, nraw, nvar, nx)) if (want_raw and nsel) else None
     res.flags = np.zeros(nmem, dtype=np.int32)
-    flags_p = res.flags.ctypes.data_as(C.POINTER(C.c_int32))
-    if name == "Classic":
-        res.final = {"E": np.empty((nmem, nx)), "Tg": np.empty((nmem, nx))}
-        out = _lib.ClassicOutputs(_lib.dptr(res.diag), _lib.dptr(res.seasonal), _lib.dptr(res.raw),
-                                  _lib.dptr(res.final["E"]), _lib.dptr(res.final["Tg"]), flags_p)
-        if multi is not None:
-            _lib.check(lib.ebm_classic_run_multi(C.byref(grid), nmem, _lib.dptr(par), _lib.dptr(forc), _lib.dptr(arrs["E"]),
-                                                 _lib.dptr(arrs["Tg"]), C.byref(opt), C.byref(multi), C.byref(out)))
-        else:
-            _lib.check(lib.ebm_classic_run(C.byref(grid), nmem, _lib.dptr(par), _lib.dptr(forc), _lib.dptr(arrs["E"]),
-                                           _lib.dptr(arrs["Tg"]), C.byref(opt), C.byref(out)))
+    finals = m.state + (("T0",) if m.T0 else ())
+    res.final = {k: np.empty((nmem, nx)) for k in finals}
+    for c in m.counters:
+        setattr(res, c, np.zeros(nmem, dtype=np.int64))
+    out = m.outputs(_lib.dptr(res.diag), _lib.dptr(res.seasonal), _lib.dptr(res.raw), *[_lib.dptr(res.final[k]) for k in finals],
+                    *[getattr(res, c).ctypes.data_as(C.POINTER(C.c_int64)) for c in m.counters],
+                    res.flags.ctypes.data_as(C.POINTER(C.c_int32)))
+    args = [C.byref(grid), nmem, _lib.dptr(par), _lib.dptr(forc), *[_lib.dptr(arrs.get(k)) for k in finals], C.byref(opt)]
+    if multi is not None:
+        _lib.check(getattr(lib, m.run_multi)(*args, C.byref(multi), C.byref(out)))
     else:
-        res.final = {k: np.empty((nmem, nx)) for k in _MIZ_STATE + ("T0",)}
-        res.newton_iters = np.zeros(nmem, dtype=np.int64)
-        res.nonconv = np.zeros(nmem, dtype=np.int64)
-        out = _lib.MizOutputs(_lib.dptr(res.diag), _lib.dptr(res.seasonal), _lib.dptr(res.raw),
-                              *[_lib.dptr(res.final[k]) for k in _MIZ_STATE + ("T0",)],
-                              res.newton_iters.ctypes.data_as(C.POINTER(C.c_int64)),
-                              res.nonconv.ctypes.data_as(C.POINTER(C.c_int64)), flags_p)
-        if multi is not None:
-            _lib.check(lib.ebm_miz_run_multi(C.byref(grid), nmem, _lib.dptr(par), _lib.dptr(forc),
-                                             *[_lib.dptr(arrs[k]) for k in _MIZ_STATE], _lib.dptr(arrs.get("T0")),
-                                             C.byref(opt), C.byref(multi), C.byref(out)))
-        else:
-            _lib.check(lib.ebm_miz_run(C.byref(grid), nmem, _lib.dptr(par), _lib.dptr(forc), *[_lib.dptr(arrs[k]) for k in _MIZ_STATE],
-                                       _lib.dptr(arrs.get("T0")), C.byref(opt), C.byref(out)))
+        _lib.check(getattr(lib, m.run)(*args, C.byref(out)))
     return res
 
 

@@ -232,6 +232,44 @@ def test_multi_gpu_entry_point_matches_single_gpu_bitwise():
     assert r.seasonal.shape == ref.seasonal.shape and _same(r.seasonal, ref.seasonal) and _same(r.raw, ref.raw)
 
 
+def test_multi_gpu_diagnostics_on_device_match_single_gpu_bitwise():
+    """ebm_miz_run_multi with the diagnostics in device memory of GPU 0 (multi.diag_device = 0): the other GPU sends
+    its rows there over NCCL.  Diagnostics, final state, counters, flags and field outputs equal the single-GPU call's
+    bit for bit.  Runs on one GPU too."""
+    import ctypes as C
+    import torch
+    from ebm_b200 import _lib
+    ndev = min(torch.cuda.device_count(), 2)
+    nmem, nx = 75, 60
+    st = ebm.SpaceTime(nx, 400, 1, "sin")
+    forcings, pars = _ensemble(nmem)
+    ref = ebm.integrate_ensemble("MIZ", st, forcings, pars, [_zero(nx) for _ in range(nmem)], field_stride=4)
+    lib = _lib.load()
+    d_diag = torch.full((nmem, 1, 3, 4), float("nan"), dtype=torch.float64, device="cuda:0")
+    seasonal, raw = np.empty_like(ref.seasonal), np.empty_like(ref.raw)
+    final = {k: np.empty((nmem, nx)) for k in STATE + ("T0",)}
+    iters, nonconv = np.zeros(nmem, dtype=np.int64), np.zeros(nmem, dtype=np.int64)
+    flags = np.zeros(nmem, dtype=np.int32)
+    i64 = C.POINTER(C.c_int64)
+    out = _lib.MizOutputs(C.cast(d_diag.data_ptr(), C.POINTER(C.c_double)), _lib.dptr(seasonal), _lib.dptr(raw),
+                          *[_lib.dptr(final[k]) for k in STATE + ("T0",)], iters.ctypes.data_as(i64),
+                          nonconv.ctypes.data_as(i64), flags.ctypes.data_as(C.POINTER(C.c_int32)))
+    par = np.array([[p[k] for k in ebm.MIZ_PAR_ORDER] for p in pars])
+    forc = np.stack([f.row() for f in forcings])
+    z = np.zeros((nmem, nx))
+    grid, opt = _lib.make_grid(st), _lib.make_options(field_stride=4)
+    multi = _lib.make_multi(devices=list(range(ndev)), diag_device=0, packet=8)
+    _lib.check(lib.ebm_miz_run_multi(C.byref(grid), nmem, _lib.dptr(par), _lib.dptr(forc), *[_lib.dptr(z)] * 5, None,
+                                     C.byref(opt), C.byref(multi), C.byref(out)))
+    torch.cuda.synchronize()
+    assert _same(d_diag.cpu().numpy(), ref.diag)
+    for k in STATE + ("T0",):
+        assert _same(final[k], ref.final[k]), k
+    assert np.array_equal(iters, ref.newton_iters) and np.array_equal(nonconv, ref.nonconv)
+    assert np.array_equal(flags, ref.flags)
+    assert _same(seasonal, ref.seasonal) and _same(raw, ref.raw)
+
+
 def test_sampler_self_consistency_and_diagnostics():
     """savesol! semantics on the device (infrastructure.jl:549-591): winter / summer snapshots are the raw steps
     winter.inx / summer.inx, the annual mean is the mean of the year's raw steps, and the L0 diagnostics equal
