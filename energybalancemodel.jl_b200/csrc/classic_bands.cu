@@ -28,11 +28,9 @@
 
 namespace {
 
-constexpr double kTwoPi = 6.283185307179586;
-
-// fast reciprocal for well-scaled operands (pivots of a diagonally dominant matrix, 1 <= |w| < 1e4):
-// MUFU.RCP64H seed + two Newton steps, ~1 ulp, no denormal/overflow slow path.
-__device__ __forceinline__ double fast_rcp(double w) {
+// reciprocal for well-scaled operands (pivots of a diagonally dominant matrix, 1 <= |w| < 1e4): MUFU.RCP64H seed +
+// two Newton steps, ~1 ulp, no denormal/overflow slow path.  Not ebm_rcp: its one cubic step gives other bits.
+__device__ __forceinline__ double rcp_newton2(double w) {
   double x;
   asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(x) : "d"(w));
   double e = fma(-w, x, 1.0);
@@ -128,10 +126,10 @@ __global__ void __launch_bounds__(MAXT, MINB) classic_bands_kernel(const Classic
   __syncthreads();
 
   const long long mo = a.orig != nullptr ? a.orig[m] : m;   // original member index: output rows
-  const bool sel = active && a.field_stride > 0 && (mo % a.field_stride) == 0;
-  const long long msel = sel ? mo / a.field_stride : 0;
-  const long long nraw = a.lastonly ? (long long)nt : (long long)nt * a.dur;
-  // Forcing{true}: base == peak == cool, all breakpoints 0 -> the call is the constant `base`
+  const bool sel = active && ebm_field_selected(a, mo);
+  const long long msel = sel ? ebm_field_row(a, mo) : 0;
+  const long long nraw = ebm_nraw(nt, a.dur, a.lastonly);
+  // Forcing{true}: the call is `base`.  Not ebm_forcing_const / _at: +5 instructions (-6 with a by-value accessor)
   const double fbase = fr[0 * MW + mi];
   const bool myconst = fr[1 * MW + mi] == fbase && fr[2 * MW + mi] == fbase && fr[6 * MW + mi] == 0.0 &&
                        fr[7 * MW + mi] == 0.0 && fr[8 * MW + mi] == 0.0 && fr[9 * MW + mi] == 0.0;
@@ -150,10 +148,9 @@ __global__ void __launch_bounds__(MAXT, MINB) classic_bands_kernel(const Classic
                              ebm_global_time(tinx, nt));
       }
       const double fmA = f - pA;
-      // savesol! branch chain (infrastructure.jl:573-588)
-      const int season = (ti == a.winter_inx) ? 0 : (ti == a.summer_inx) ? 1 : (ti == nt) ? 2 : -1;
-      const bool rawstep = sel && a.raw != nullptr && (!a.lastonly || year == a.dur - 1);
-      const long long rawidx = a.lastonly ? (ti - 1) : ((long long)year * nt + ti - 1);
+      const int season = ebm_season(a, ti, nt);
+      const bool rawstep = sel && a.raw != nullptr && ebm_raw_year(year, a.dur, a.lastonly);
+      const long long rawidx = ebm_raw_slot(year, ti, nt, a.lastonly);
 
       double q[K], s[K];  // Tg[] is reused for rhs -> y -> solution
       double dgT = 0.0, dgE = 0.0, dgA = 0.0, dgX = 2.0;  // diagnostic partials (edge: 2.0 = none)
@@ -206,12 +203,12 @@ __global__ void __launch_bounds__(MAXT, MINB) classic_bands_kernel(const Classic
           dgE = fma(wj, vE, dgE);
           if (vE < 0.0 && j < nx) { dgA += wj; dgX = fmin(dgX, xj); }
           if (sel && a.seasonal != nullptr && j < nx) {
-            double* o = a.seasonal + ((((msel * a.dur + year) * 3 + season) * 3) * (long long)nx) + j;
+            double* o = a.seasonal + ebm_seasonal_offset(msel, a.dur, year, season, EBM_CLASSIC_NVAR, nx) + j;
             o[0] = vE; o[nx] = vT; o[2 * nx] = -vN * inv_Lf;
           }
         }
         if (rawstep && j < nx) {
-          double* o = a.raw + ((msel * nraw + rawidx) * 3) * (long long)nx + j;
+          double* o = a.raw + ebm_raw_offset(msel, nraw, rawidx, EBM_CLASSIC_NVAR, nx) + j;
           o[0] = En; o[nx] = T; o[2 * nx] = -Eneg * inv_Lf;   // h = -E/Lf*(E<0)  (:65)
         }
         if (ti == nt) { sumE[sidx] = 0.0; sumT[sidx] = 0.0; sumH[sidx] = 0.0; }
@@ -235,7 +232,7 @@ __global__ void __launch_bounds__(MAXT, MINB) classic_bands_kernel(const Classic
         const double ai_ = -fac * lamlo[j];
         const double ci_ = -fac * lamhi[j];
         const double w = (i == 0) ? diag : fma(-ai_, qprev, diag);
-        const double iw = fast_rcp(w);
+        const double iw = rcp_newton2(w);
         const double tq = ai_ * iw;
         q[i] = ci_ * iw;
         const double yi = (i == 0) ? rhs * iw : fma(-tq, yprev, rhs * iw);
@@ -275,7 +272,7 @@ __global__ void __launch_bounds__(MAXT, MINB) classic_bands_kernel(const Classic
             rh = fma(-ql, n6[3 * MW], yl);
           }
           const double w = (b == 0) ? dg : fma(-sl, cq, dg);
-          const double iw = fast_rcp(w);
+          const double iw = rcp_newton2(w);
           cy = (b == 0) ? rh * iw : fma(-sl, cy, rh) * iw;
           cq = sup * iw;
           cqs[b * MW + mi] = cq; cys[b * MW + mi] = cy;
@@ -292,8 +289,7 @@ __global__ void __launch_bounds__(MAXT, MINB) classic_bands_kernel(const Classic
             const double* r4 = red + (b * 4) * MW + mi;
             t0 += r4[0 * MW]; t1 += r4[1 * MW]; t2 += r4[2 * MW]; t3 = fmin(t3, r4[3 * MW]);
           }
-          double* o = a.diag + ((mo * a.dur + year) * 3 + season) * 4;
-          o[0] = t0; o[1] = t1; o[2] = kTwoPi * t2; o[3] = (t3 > 1.5) ? 1.0 : t3;
+          ebm_store_diag(a.diag, mo, a.dur, year, season, t0, t1, t2, t3);
         }
       }
       __syncthreads();
@@ -319,7 +315,7 @@ __global__ void __launch_bounds__(MAXT, MINB) classic_bands_kernel(const Classic
     if (j < nx && active) {
       a.E[(long long)j * nmem + m] = E[i];
       a.Tg[(long long)j * nmem + m] = Tg[i];
-      bad = bad || !(fabs(E[i]) < 1e300) || !(fabs(Tg[i]) < 1e300);
+      bad = bad || ebm_state_bad(E[i]) || ebm_state_bad(Tg[i]);
     }
   }
   if (bad && a.flags != nullptr) atomicOr(a.flags + mo, 1);

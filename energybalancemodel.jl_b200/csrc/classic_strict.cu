@@ -9,8 +9,6 @@
 
 namespace {
 
-constexpr double kPi = 3.141592653589793;
-
 struct Lit {  // literal IEEE ops, never contracted
   static __device__ __forceinline__ double add(double a, double b) { return __dadd_rn(a, b); }
   static __device__ __forceinline__ double sub(double a, double b) { return __dsub_rn(a, b); }
@@ -120,27 +118,23 @@ __global__ void classic_strict_kernel(const ClassicKArgs a, double* ws) {
   const double Lf = p[12 * nmem];
   const double* fr = a.forc + m;
   const long long mo = a.orig != nullptr ? a.orig[m] : m;   // original member index: output rows
-  const bool sel = a.field_stride > 0 && (mo % a.field_stride) == 0;
-  const long long msel = sel ? mo / a.field_stride : 0;
-  const long long nraw = a.lastonly ? (long long)nt : (long long)nt * a.dur;
+  const bool sel = ebm_field_selected(a, mo);
+  const long long msel = sel ? ebm_field_row(a, mo) : 0;
+  const long long nraw = ebm_nraw(nt, a.dur, a.lastonly);
   for (int j = 0; j < nx; ++j) { sE[j * nmem] = 0.0; sT[j * nmem] = 0.0; sH[j * nmem] = 0.0; }
 
   for (int year = a.year0; year < a.year0 + a.nyears; ++year) {
     for (int ti = 1; ti <= nt; ++ti) {
-      const long long tinx = (long long)year * nt + ti;
-      const double f = ebm_forcing_eval(fr[0], fr[1 * nmem], fr[2 * nmem], fr[3 * nmem], fr[4 * nmem], fr[6 * nmem],
-                                        fr[7 * nmem], fr[8 * nmem], fr[9 * nmem],
-                                        ebm_global_time(tinx + (long long)a.start_year * nt, nt));
+      const double f = ebm_forcing_at([&](int r) { return fr[r * nmem]; }, (long long)(year + a.start_year) * nt + ti, nt);
       classic_step_literal(a.g, p, nmem, s, ti, f, E, Tg, Tc, dg, y, w, nmem);
       for (int j = 0; j < nx; ++j) {
         const double Ej = E[j * nmem];
         sE[j * nmem] += Ej; sT[j * nmem] += Tc[j * nmem];
         sH[j * nmem] += (Ej < 0.0 ? Lit::div(-Ej, Lf) : 0.0);
       }
-      const int season = (ti == a.winter_inx) ? 0 : (ti == a.summer_inx) ? 1 : (ti == nt) ? 2 : -1;
-      if (sel && a.raw != nullptr && (!a.lastonly || year == a.dur - 1)) {
-        const long long rawidx = a.lastonly ? (ti - 1) : (tinx - 1);
-        double* o = a.raw + ((msel * nraw + rawidx) * 3) * (long long)nx;
+      const int season = ebm_season(a, ti, nt);
+      if (sel && a.raw != nullptr && ebm_raw_year(year, a.dur, a.lastonly)) {
+        double* o = a.raw + ebm_raw_offset(msel, nraw, ebm_raw_slot(year, ti, nt, a.lastonly), EBM_CLASSIC_NVAR, nx);
         for (int j = 0; j < nx; ++j) {
           const double Ej = E[j * nmem];
           o[j] = Ej; o[nx + j] = Tc[j * nmem]; o[2 * nx + j] = Ej < 0.0 ? Lit::div(-Ej, Lf) : 0.0;  // :65
@@ -157,17 +151,14 @@ __global__ void classic_strict_kernel(const ClassicKArgs a, double* ws) {
           return Ej < 0.0 ? Lit::div(-Ej, Lf) : 0.0;
         };
         if (sel && a.seasonal != nullptr) {
-          double* o = a.seasonal + (((msel * a.dur + year) * 3 + season) * 3) * (long long)nx;
+          double* o = a.seasonal + ebm_seasonal_offset(msel, a.dur, year, season, EBM_CLASSIC_NVAR, nx);
           for (int j = 0; j < nx; ++j) { o[j] = vE(j); o[nx + j] = vT(j); o[2 * nx + j] = vH(j); }
         }
         if (a.diag != nullptr) {
-          double edge = 1.0; bool found = false;
-          for (int j = 0; j < nx && !found; ++j) if (vE(j) < 0.0) { edge = a.g.x[j]; found = true; }
-          double* o = a.diag + ((mo * a.dur + year) * 3 + season) * 4;
-          o[0] = hemi_mean(a.g.x, nx, vT);
-          o[1] = hemi_mean(a.g.x, nx, vE);
-          o[2] = Lit::mul(Lit::mul(2.0, kPi), hemi_mean(a.g.x, nx, [&](int j) { return vE(j) < 0.0 ? 1.0 : 0.0; }));
-          o[3] = edge;
+          double edge = 2.0;   // no ice
+          for (int j = 0; j < nx; ++j) if (vE(j) < 0.0) { edge = a.g.x[j]; break; }
+          ebm_store_diag(a.diag, mo, a.dur, year, season, hemi_mean(a.g.x, nx, vT), hemi_mean(a.g.x, nx, vE),
+                         hemi_mean(a.g.x, nx, [&](int j) { return vE(j) < 0.0 ? 1.0 : 0.0; }), edge);
         }
       }
       if (ti == nt) for (int j = 0; j < nx; ++j) { sE[j * nmem] = 0.0; sT[j * nmem] = 0.0; sH[j * nmem] = 0.0; }
@@ -175,7 +166,7 @@ __global__ void classic_strict_kernel(const ClassicKArgs a, double* ws) {
   }
   if (a.flags != nullptr) {
     bool bad = false;
-    for (int j = 0; j < nx; ++j) bad = bad || !(fabs(E[j * nmem]) < 1e300) || !(fabs(Tg[j * nmem]) < 1e300);
+    for (int j = 0; j < nx; ++j) bad = bad || ebm_state_bad(E[j * nmem]) || ebm_state_bad(Tg[j * nmem]);
     if (bad) atomicOr(a.flags + mo, 1);
   }
 }

@@ -49,20 +49,10 @@ __device__ unsigned long long g_phase_cycles[8][8];
 
 namespace {
 
-constexpr double kTwoPi = 6.283185307179586;
-
-// reciprocal for well-scaled operands: MUFU.RCP64H seed + one cubic step (~1 ulp, no slow path)
-__device__ __forceinline__ double fast_rcp(double w) {
-  // the seed is good to 2^-20 (measured, profiles/r2_microbench.txt): one cubic step reaches 1 ulp
-  double x;
-  asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(x) : "d"(w));
-  const double e = fma(-w, x, 1.0);
-  const double t = fma(e, e, e);
-  return fma(x, t, x);
-}
-// sign tests on the high word (integer pipe, not the FP64 pipe).  The state never holds -0.0: it is normalised when
+// sign test on the high word (integer pipe, not the FP64 pipe).  The state never holds -0.0: it is normalised when
 // loaded, and E + dt*(...) cannot produce it (an exact cancellation rounds to +0.0).
 __device__ __forceinline__ bool is_neg(double v) { return __double2hiint(v) < 0; }
+// (miz_kernel.cu's is_zero, the same predicate in another form, changes the code of every instance: -46 to -168 instructions)
 __device__ __forceinline__ bool is_zero(double v) { return ((__double2hiint(v) << 1) | __double2loint(v)) == 0; }
 
 struct __align__(16) PhysTab { double S0x, S1x, aw, wts; };      // per cell
@@ -150,12 +140,12 @@ struct Ctx {
       const int sidx = cidx(i);
       const double Eneg = is_neg(En) ? En : 0.0;
       if (cta_fields) { sumT[sidx] += T; sumH[sidx] += Eneg; }
-      const bool rawstep = sel && a.raw != nullptr && (!a.lastonly || year == a.dur - 1);
+      const bool rawstep = sel && a.raw != nullptr && (!a.lastonly || year == a.dur - 1);   // not ebm_raw_year: -93 to +84 instr.
       if (rawstep && j < nx) {
-        const long long nraw = a.lastonly ? (long long)nt : (long long)nt * a.dur;
-        const long long rawidx = a.lastonly ? (ti - 1) : ((long long)year * nt + ti - 1);
-        const long long msel = member_orig(a) / a.field_stride;
-        double* o = a.raw + ((msel * nraw + rawidx) * 3) * (long long)nx + j;
+        const long long nraw = ebm_nraw(nt, a.dur, a.lastonly);   // (this order of loads keeps the code)
+        const long long slot = ebm_raw_slot(year, ti, nt, a.lastonly);
+        const long long msel = ebm_field_row(a, member_orig(a));
+        double* o = a.raw + ebm_raw_offset(msel, nraw, slot, EBM_CLASSIC_NVAR, nx) + j;
         o[0] = En; o[nx] = T; o[2 * nx] = -Eneg * inv_Lf;          // h = -E/Lf*(E<0)  (classic.jl:65)
       }
       if (season >= 0) {
@@ -168,8 +158,8 @@ struct Ctx {
         dgE = fma(wj, vE, dgE);
         if (vE < 0.0 && j < nx) { dgA += wj; dgX = fmin(dgX, phys[j].S1x); }
         if (sel && a.seasonal != nullptr && j < nx) {
-          const long long msel = member_orig(a) / a.field_stride;
-          double* o = a.seasonal + ((((msel * a.dur + year) * 3 + season) * 3) * (long long)nx) + j;
+          const long long msel = ebm_field_row(a, member_orig(a));
+          double* o = a.seasonal + ebm_seasonal_offset(msel, a.dur, year, season, EBM_CLASSIC_NVAR, nx) + j;
           o[0] = vE; o[nx] = vT; o[2 * nx] = -vN * inv_Lf;
         }
       }
@@ -198,7 +188,7 @@ struct Ctx {
       for (int i = 0; i < K; ++i) {
         if (i >= nv) {
           E[i] = wantice ? -10.0 : 100.0; Tg[i] = wantice ? -10.0 : 10.0;
-          rs.r(i) = E[i] * fast_rcp(fma(M, E[i], -kLf));
+          rs.r(i) = E[i] * ebm_rcp(fma(M, E[i], -kLf));
         }
       }
     }
@@ -337,7 +327,7 @@ struct Ctx {
     const int nx = a.nx, nt = a.nt;
     const double fmA = f - A;
     const double fmAFb = fmA + Fb;
-    const int season = SLOW ? ((ti == a.winter_inx) ? 0 : (ti == a.summer_inx) ? 1 : (ti == nt) ? 2 : -1) : -1;
+    const int season = SLOW ? ebm_season(a, ti, nt) : -1;
     // rs.q(i): dt_tau/(M - kLf/E) of a masked row (else 0): the diagonal decrement over cg_tau; later the pivots / spikes
     bool anymask = !TAB;   // without precomputed pivots every band eliminates in full
     PHASE_BEGIN();
@@ -388,7 +378,7 @@ struct Ctx {
             const double Eo = fma(-dt, Cb, En) / fma(-dt * M, inv_cw, 1.0);
             const double C = Cb - Fb;
             const double T0 = C / (M - kLf / Eo);                                                 //     :50
-            const double r = En * fast_rcp(fma(M, En, -kLf));
+            const double r = En * ebm_rcp(fma(M, En, -kLf));
             rs.r(i) = r;
             if (T0 < 0.0) {
               rs.q(i) = dt_tau * r; anymask = true;
@@ -442,7 +432,7 @@ struct Ctx {
         const CoefTab cf = coef_at(j0 + i);
         const double diag = fma(-cg_tau, rs.q(i), cf.kjj);      // kappa_jj - dc/(M - kLf/E) [masked]   :56
         const double P = (i == 0) ? diag : fma(diag, Pm1, -(cf.ac * Pm2));
-        rs.s(i) = Pm1 * fast_rcp(P);            // 1 / w_i
+        rs.s(i) = Pm1 * ebm_rcp(P);            // 1 / w_i
         Pm2 = Pm1; Pm1 = P;
       }
       double yprev = 0.0, sprev = 0.0;
@@ -503,7 +493,7 @@ struct Ctx {
       double cq[H], cy[H];
 #pragma unroll
       for (int k = 0; k < H; ++k) {
-        const double iw = Dm[k] * fast_rcp(Dm[k + 1]);
+        const double iw = Dm[k] * ebm_rcp(Dm[k + 1]);
         cq[k] = c_[k] * iw;
         const double g = a_[k] * iw, ri = r_[k] * iw;
         cy[k] = (k == 0) ? ri : fma(-g, cy[k - 1], ri);
@@ -511,7 +501,7 @@ struct Ctx {
       // the two sweeps meet between rows H-1 and H:  x_own = cy_own - cq_own * x_other
       const double ocq = __shfl_xor_sync(0xffffffffu, cq[H - 1], MW);
       const double ocy = __shfl_xor_sync(0xffffffffu, cy[H - 1], MW);
-      double x = fma(-cq[H - 1], ocy, cy[H - 1]) * fast_rcp(fma(-cq[H - 1], ocq, 1.0));
+      double x = fma(-cq[H - 1], ocy, cy[H - 1]) * ebm_rcp(fma(-cq[H - 1], ocq, 1.0));
       zs[(half ? (WB - H) : (H - 1)) * MW + mi] = x;
 #pragma unroll
       for (int k = H - 2; k >= 0; --k) {
@@ -525,8 +515,7 @@ struct Ctx {
           t1 += r4[1 * MW]; t2 += r4[2 * MW]; t3 = fmin(t3, r4[3 * MW]);
           t0 += r4[0 * MW];
         }
-        double* o = a.diag + ((member_orig(a) * a.dur + year) * 3 + season) * 4;
-        o[0] = t0; o[1] = t1; o[2] = kTwoPi * t2; o[3] = (t3 > 1.5) ? 1.0 : t3;
+        ebm_store_diag(a.diag, member_orig(a), a.dur, year, season, t0, t1, t2, t3);
       }
     }
     PHASE_MARK(3);   // interface solve (warp 0) / nothing
@@ -677,7 +666,7 @@ __global__ void __maxnreg__(MAXR) classic_uniform_kernel(const __grid_constant__
   cx.solver = (a.dbg & 8) ? warp == 0 : (wrot == (NWARP > 1 ? 1 : 0));
   cx.active = active;
   const long long mo = a.orig != nullptr ? a.orig[m] : m;   // ebm_classic_device_args_t.member_index
-  cx.sel = active && a.field_stride > 0 && (mo % a.field_stride) == 0;
+  cx.sel = active && ebm_field_selected(a, mo);
   cx.cta_fields = __syncthreads_or(cx.sel && (a.seasonal != nullptr)) != 0;
   cx.accT = 0.0;
 #pragma unroll
@@ -689,21 +678,19 @@ __global__ void __maxnreg__(MAXR) classic_uniform_kernel(const __grid_constant__
     cx.E[i] = (v ? a.E[(long long)j * nmem + m] : 1.0) + 0.0;     // pad cells: decoupled open-water rows
     cx.Tg[i] = v ? a.Tg[(long long)j * nmem + m] : 0.0;
     sumE[cx.cidx(i)] = 0.0;
-    cx.rs.r(i) = cx.E[i] * fast_rcp(fma(cM, cx.E[i], -ckLf));   // same expression as in the step: r is a pure function of E
+    cx.rs.r(i) = cx.E[i] * ebm_rcp(fma(cM, cx.E[i], -ckLf));   // same expression as in the step: r is a pure function of E
     if (cx.cta_fields) { sumT[cx.cidx(i)] = 0.0; sumH[cx.cidx(i)] = 0.0; }
   }
   cx.set_pads(a);
-  // Forcing{true}: base == peak == cool, all breakpoints 0 -> the call is the constant `base`
-  const double fbase = fr[0 * MW + mi];
-  const bool myconst = fr[1 * MW + mi] == fbase && fr[2 * MW + mi] == fbase && fr[6 * MW + mi] == 0.0 &&
-                       fr[7 * MW + mi] == 0.0 && fr[8 * MW + mi] == 0.0 && fr[9 * MW + mi] == 0.0;
-  const bool constf = __syncthreads_and(myconst) != 0;
+  const auto frow = [&](int r) { return fr[r * MW + mi]; };
+  const double fbase = frow(0);
+  const bool constf = __syncthreads_and(ebm_forcing_const(frow)) != 0;
   const bool has_raw = __syncthreads_or(cx.sel && (a.raw != nullptr)) != 0;
 
   const double cS1 = UPAR ? a.u.par[5] : pS1;
   double S1c_next = cS1 * __ldg(a.g.ctab);   // S1*cos(2*pi*t_1); ctab[nt] == ctab[0] closes the year (classic.jl:25)
   for (int year = a.year0; year < a.year0 + a.nyears; ++year) {
-    const bool raw_year = has_raw && (!a.lastonly || year == a.dur - 1);
+    const bool raw_year = has_raw && (!a.lastonly || year == a.dur - 1);   // not ebm_raw_year: -3 instructions each instance
 #pragma unroll 1
     for (int ti = 1; ti <= nt; ++ti) {
       // The loop carries `ti` and `year` only: an opaque copy of the index keeps ptxas from expanding it into 64-bit
@@ -717,9 +704,7 @@ __global__ void __maxnreg__(MAXR) classic_uniform_kernel(const __grid_constant__
       double f = fbase;
       if (!constf) {
         const long long tinx = (long long)(year + a.start_year) * nt + tix;
-        f = ebm_forcing_eval(fr[0 * MW + mi], fr[1 * MW + mi], fr[2 * MW + mi], fr[3 * MW + mi], fr[4 * MW + mi],
-                             fr[6 * MW + mi], fr[7 * MW + mi], fr[8 * MW + mi], fr[9 * MW + mi],
-                             ebm_global_time(tinx, nt));
+        f = ebm_forcing_at(frow, tinx, nt);
       }
       const bool slow = cx.cta_fields || raw_year || ti == a.winter_inx || ti == a.summer_inx || ti == nt;
       if (slow) cx.template step<true>(a, f, S1c0, S1c1, ti, year);
@@ -734,7 +719,7 @@ __global__ void __maxnreg__(MAXR) classic_uniform_kernel(const __grid_constant__
     if (j < nx && active) {
       a.E[(long long)j * nmem + m] = cx.E[i];
       a.Tg[(long long)j * nmem + m] = cx.Tg[i];
-      bad = bad || !(fabs(cx.E[i]) < 1e300) || !(fabs(cx.Tg[i]) < 1e300);
+      bad = bad || ebm_state_bad(cx.E[i]) || ebm_state_bad(cx.Tg[i]);
     }
   }
   if (bad && a.flags != nullptr) atomicOr(a.flags + mo, 1);

@@ -55,8 +55,6 @@ unsigned long long fnv1a(const void* p, size_t n, unsigned long long h = 1469598
   return h;
 }
 
-constexpr double kPi = 3.141592653589793;  // Float64(pi)
-
 int check_grid(const ebm_grid_t* g) {
   if (!g || !g->x || !g->t) { ebm_set_error("grid, grid->x and grid->t must be non-NULL"); return EBM_ERR_INVALID; }
   if (g->nx < 3 || g->nt < 1 || g->dur < 1) { ebm_set_error("need nx >= 3, nt >= 1, dur >= 1 (got %d, %d, %d)", g->nx, g->nt, g->dur); return EBM_ERR_INVALID; }
@@ -232,8 +230,6 @@ int download_transposed(double* host, double* stage, const double* src, long lon
   return EBM_OK;
 }
 
-long long nsel_of(long long nmem, int stride) { return stride > 0 ? (nmem + stride - 1) / stride : 0; }
-
 // The classic kernels: the literal-order one on request; up to kClassicUniformMaxNx cells the table-driven kernel
 // (the 32-member groups whose table-building parameters agree) and its per-member-coefficient instance (the other
 // groups); larger grids the band kernel.
@@ -348,8 +344,7 @@ int ebm_run_host(const ebm_grid_t* grid, long long nmem, const EbmHostRun& run, 
   EBM_TRY(select_device(opt));
   if ((run.seasonal || run.raw) && opt.field_stride <= 0) { ebm_set_error("seasonal/raw output requested but field_stride == 0"); return EBM_ERR_INVALID; }
   const int nx = grid->nx, nt = grid->nt, dur = grid->dur;
-  const long long nsel = nsel_of(nmem, opt.field_stride);
-  const long long nraw = opt.lastonly ? nt : (long long)nt * dur;
+  const long long nsel = ebm_nsel(opt, nmem), nraw = ebm_nraw(nt, dur, opt.lastonly);
   const std::vector<long long> perm = run.order ? run.order(grid, nmem, run, opt) : std::vector<long long>();
   cudaStream_t s;
   EBM_CUDA_TRY(cudaStreamCreate(&s));
@@ -386,9 +381,9 @@ int ebm_run_host(const ebm_grid_t* grid, long long nmem, const EbmHostRun& run, 
     dev.init[q] = dev.fin[q];
   }
   // outputs: allocated when wanted; fields and diagnostics NaN (what the reference leaves undef), counters zero
-  const size_t ndiag = (size_t)nmem * dur * EBM_NSEASON * EBM_NDIAG;
-  const size_t nseas = (size_t)nsel * dur * EBM_NSEASON * run.nvar * nx;
-  const size_t nrawn = (size_t)nsel * nraw * run.nvar * nx;
+  const size_t ndiag = ebm_diag_offset(nmem, dur, 0, 0);
+  const size_t nseas = ebm_seasonal_offset(nsel, dur, 0, 0, run.nvar, nx);
+  const size_t nrawn = ebm_raw_offset(nsel, nraw, 0, run.nvar, nx);
   auto nan_filled = [&](double** d, bool wanted, size_t n) -> int {
     *d = nullptr;
     if (!wanted) return EBM_OK;

@@ -157,7 +157,54 @@ int ebm_launch_gather_transpose(const double* src, double* dst, long long rows, 
 int ebm_run_fp64_peak(int device, double* tflops, double* mhz);
 
 // ----------------------------------------------------------------------------- small device helpers
-// Forcing call (src/infrastructure.jl:294-307).  fr = base, peak, cool, rate_up, rate_down, d1..d5.
+constexpr double kPi = 3.141592653589793;   // Float64(pi)
+constexpr unsigned kFull = 0xffffffffu;
+#define EBM_HD __host__ __device__ __forceinline__
+
+// ---- output layout (include/ebm_cuda.h).  Every offset is in doubles from the start of its array; the offset of
+// member (or row) n, all other indices 0, is the length of n members' records.
+// The helpers that take `o` (ebm_options_t or a kernel argument block) read its fields only where the expression needs
+// them: arguments evaluated up front change the generated code of the production classic kernels.
+// Field output (seasonal, raw) is kept for every field_stride-th member (original index), in row m / field_stride.
+template <class Opt>
+EBM_HD bool ebm_field_selected(const Opt& o, long long m) { return o.field_stride > 0 && (m % o.field_stride) == 0; }
+template <class Opt> EBM_HD long long ebm_field_row(const Opt& o, long long m) { return m / o.field_stride; }
+template <class Opt>
+EBM_HD long long ebm_nsel(const Opt& o, long long nmem) {
+  return o.field_stride > 0 ? (nmem + o.field_stride - 1) / o.field_stride : 0;
+}
+// Raw fields: every step of the run, or with lastonly every step of its last year; slot of step ti (1-based) of year
+EBM_HD long long ebm_nraw(int nt, int dur, int lastonly) { return lastonly ? (long long)nt : (long long)nt * dur; }
+EBM_HD bool ebm_raw_year(int year, int dur, int lastonly) { return !lastonly || year == dur - 1; }
+EBM_HD long long ebm_raw_slot(int year, int ti, int nt, int lastonly) {
+  return lastonly ? (ti - 1) : ((long long)year * nt + ti - 1);
+}
+// raw [nsel][nraw][nvar][nx], seasonal [nsel][dur][EBM_NSEASON][nvar][nx], diag [nmem][dur][EBM_NSEASON][EBM_NDIAG]
+EBM_HD long long ebm_raw_offset(long long msel, long long nraw, long long slot, int nvar, int nx) {
+  return ((msel * nraw + slot) * nvar) * (long long)nx;
+}
+EBM_HD long long ebm_seasonal_offset(long long msel, int dur, int year, int season, int nvar, int nx) {
+  return (((msel * dur + year) * 3 + season) * nvar) * (long long)nx;
+}
+EBM_HD long long ebm_diag_offset(long long m, int dur, int year, int season) { return ((m * dur + year) * 3 + season) * 4; }
+// One diagnostics record: hemispheric means of T and E, ice area (hemispheric mean of the ice mask, times 2 pi) and
+// ice edge.  edge > 1.5 means no ice: the edge is then 1.
+__device__ __forceinline__ void ebm_store_diag(double* diag, long long m, int dur, int year, int season, double meanT,
+                                               double meanE, double area, double edge) {
+  double* o = diag + ebm_diag_offset(m, dur, year, season);
+  o[0] = meanT; o[1] = meanE; o[2] = 2.0 * kPi * area; o[3] = (edge > 1.5) ? 1.0 : edge;
+}
+
+// savesol! (infrastructure.jl:573-588): the season step ti samples -- 0 winter, 1 summer, 2 annual mean (the
+// year's last step), -1 none.  a: the kernel argument block; nt: a.nt as the caller holds it
+template <class KArgs>
+__device__ __forceinline__ int ebm_season(const KArgs& a, int ti, int nt) {
+  return (ti == a.winter_inx) ? 0 : (ti == a.summer_inx) ? 1 : (ti == nt) ? 2 : -1;
+}
+
+// ---- forcing.  fr(r) returns row r of the member's forcing (base, peak, cool, rate_up, rate_down, d1..d5), from
+// wherever the kernel keeps it; row 5 (d1) is not read.
+// Forcing call (src/infrastructure.jl:294-307)
 __device__ __forceinline__ double ebm_forcing_eval(double base, double peak, double cool, double rup, double rdown,
                                                    double d2, double d3, double d4, double d5, double T) {
   if (T < d2) return base;
@@ -166,10 +213,46 @@ __device__ __forceinline__ double ebm_forcing_eval(double base, double peak, dou
   if (T < d5) return peak + rdown * (T - d4);
   return cool;
 }
-
 // SpaceTime.T[tinx] (1-based): correctly rounded (2*tinx-1)/(2*nt)  (infrastructure.jl:130, TwicePrecision range)
 __device__ __forceinline__ double ebm_global_time(long long tinx, int nt) {
   return __ddiv_rn((double)(2 * tinx - 1), (double)(2LL * nt));
+}
+// the call at global step tinx (1-based, counted over every year simulated)
+template <class Fr>
+__device__ __forceinline__ double ebm_forcing_at(Fr fr, long long tinx, int nt) {
+  return ebm_forcing_eval(fr(0), fr(1), fr(2), fr(3), fr(4), fr(6), fr(7), fr(8), fr(9), ebm_global_time(tinx, nt));
+}
+// Forcing{true}: base == peak == cool and the breakpoints d2..d5 are 0, so every call returns `base`
+template <class Fr>
+__device__ __forceinline__ bool ebm_forcing_const(Fr fr) {
+  return fr(1) == fr(0) && fr(2) == fr(0) && fr(6) == 0.0 && fr(7) == 0.0 && fr(8) == 0.0 && fr(9) == 0.0;
+}
+
+// A final state value the run cannot continue from: NaN, +-Inf or |v| >= 1e300 (flags bit 0)
+__device__ __forceinline__ bool ebm_state_bad(double v) { return !(fabs(v) < 1e300); }
+
+// ---- arithmetic
+// Reciprocal of an ordinary number (normal, 2^-1000 < |y| < 2^1000): MUFU.RCP64H seed, good to 2^-20 (measured,
+// profiles/r2_microbench.txt), and one cubic step (3 FMA): ~1 ulp, no slow path
+__device__ __forceinline__ double ebm_rcp(double y) {
+  double r;
+  asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(y));
+  const double e = fma(-y, r, 1.0);
+  return fma(r, fma(e, e, e), r);
+}
+
+// ---- one warp = one member (MIZ)
+__device__ __forceinline__ double ebm_shfl_up1(double v) { return __shfl_up_sync(kFull, v, 1); }
+__device__ __forceinline__ double ebm_shfl_dn1(double v) { return __shfl_down_sync(kFull, v, 1); }
+__device__ __forceinline__ double ebm_warp_sum(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(kFull, v, o);
+  return v;
+}
+__device__ __forceinline__ double ebm_warp_min(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(kFull, v, o));
+  return v;
 }
 
 // The classic parameters that feed the CTA-wide tables of classic_uniform.cu: D, cg, tau (the matrix kappa,

@@ -189,10 +189,10 @@ struct GatherHook : EbmDiagHook {
 // global index / field_stride in the caller's arrays.
 struct FieldSel {
   std::vector<long long> member, slot;   // the member's index, its row in the caller's field arrays
-  FieldSel(const std::vector<long long>& ix, int stride, bool wanted) {
-    if (!wanted || stride <= 0) return;
+  FieldSel(const std::vector<long long>& ix, const ebm_options_t& opt, bool wanted) {
+    if (!wanted) return;
     for (long long m : ix)
-      if (m % stride == 0) { member.push_back(m); slot.push_back(m / stride); }
+      if (ebm_field_selected(opt, m)) { member.push_back(m); slot.push_back(ebm_field_row(opt, m)); }
   }
   bool any() const { return !member.empty(); }
 };
@@ -265,7 +265,7 @@ int run_multi(const ebm_grid_t* grid, long long nmem, const EbmHostRun& run, con
   int rc = resolve_devices(multi, &devs);
   if (rc != EBM_OK) return rc;
   const int ndev = (int)devs.size(), nx = grid->nx;
-  const size_t rowlen = (size_t)grid->dur * EBM_NSEASON * EBM_NDIAG;
+  const size_t rowlen = ebm_diag_offset(1, grid->dur, 0, 0);
   NcclGather g;
   g.idx = deal(nmem, ndev, key, (multi && multi->packet > 0) ? multi->packet : 32);
   const int nccl = setup_gather(multi, devs, &g, run.diag, rowlen);
@@ -303,10 +303,11 @@ int run_multi(const ebm_grid_t* grid, long long nmem, const EbmHostRun& run, con
     put_rows(run.newton_iters, it, ix, 1);
     put_rows(run.nonconv, nc, ix, 1);
     put_rows(run.flags, fl, ix, 1);
-    const FieldSel fs(ix, opt_in ? opt_in->field_stride : 0, run.seasonal || run.raw);
+    const FieldSel fs(ix, opt_in ? *opt_in : default_options(), run.seasonal || run.raw);
     if (fs.any()) {
-      const size_t ns = fs.member.size(), nraw = (size_t)(op.lastonly ? grid->nt : (long long)grid->nt * grid->dur);
-      const size_t lenS = (size_t)grid->dur * EBM_NSEASON * run.nvar * nx, lenR = nraw * run.nvar * nx;
+      const size_t ns = fs.member.size();
+      const size_t lenS = ebm_seasonal_offset(1, grid->dur, 0, 0, run.nvar, nx);
+      const size_t lenR = ebm_raw_offset(1, ebm_nraw(grid->nt, grid->dur, op.lastonly), 0, run.nvar, nx);
       MemberRows in2;
       EbmHostRun r2 = members(run, fs.member, nx, &in2);
       std::vector<double> se(run.seasonal ? ns * lenS : 0), rw(run.raw ? ns * lenR : 0);

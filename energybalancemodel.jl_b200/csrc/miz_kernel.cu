@@ -35,32 +35,9 @@
 
 namespace {
 
-constexpr double kPi = 3.141592653589793;   // Float64(pi)
-constexpr unsigned kFull = 0xffffffffu;
 constexpr int kWarps = 4;                   // members per CTA
 constexpr int kGC = 3;                      // cells per statement-major group when K allows it (DESIGN.md 4.3)
 
-__device__ __forceinline__ double shfl_up1(double v) { return __shfl_up_sync(kFull, v, 1); }
-__device__ __forceinline__ double shfl_dn1(double v) { return __shfl_down_sync(kFull, v, 1); }
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(kFull, v, o);
-  return v;
-}
-__device__ __forceinline__ double warp_min(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(kFull, v, o));
-  return v;
-}
-
-// reciprocal of an ordinary number (normal, 2^-1000 < |y| < 2^1000): ~1 ulp, no slow path.  The MUFU.RCP64H seed is
-// good to 2^-20 (measured, profiles/r2_microbench.txt): one cubic step (3 FMA) reaches 1 ulp
-__device__ __forceinline__ double rcp_nr(double y) {
-  double r;
-  asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(y));
-  const double e = fma(-y, r, 1.0);
-  return fma(r, fma(e, e, e), r);
-}
 // c ? a : b as one SELP with both operands evaluated: the compiler otherwise branches around "expensive" operands,
 // which splits the unrolled per-cell code into scheduling regions and serialises the K cells of a lane
 __device__ __forceinline__ double keep(double v) {
@@ -84,11 +61,11 @@ __device__ __forceinline__ double sel1(bool c, double b) {
 // zero / sign tests on the integer pipe (the FP64 pipe is the bottleneck); +0 and -0 are both zero
 __device__ __forceinline__ bool is_zero(double v) { return ((__double2hiint(v) & 0x7fffffff) | __double2loint(v)) == 0; }   // one LOP3 with predicate output
 // x / y with y an ordinary non-zero number (no denormal / huge denominators: DESIGN.md 4.3)
-__device__ __forceinline__ double div_n(double x, double y) { return x * rcp_nr(y); }
+__device__ __forceinline__ double div_n(double x, double y) { return x * ebm_rcp(y); }
 // x / y with y zero or ordinary: IEEE results for y == +-0 (x/0 = +-Inf, 0/0 = NaN/0 = NaN), branch free
 __device__ __forceinline__ double div_z(double x, double y) {
   const bool z = is_zero(y);
-  const double q = x * rcp_nr(sel1(z, y));
+  const double q = x * ebm_rcp(sel1(z, y));
   const double inf = __hiloint2double(0x7ff00000 | ((__double2hiint(x) ^ __double2hiint(y)) & 0x80000000), 0);
   const double zq = (is_zero(x) || x != x) ? __longlong_as_double(0x7ff8000000000000LL) : inf;
   return sel(z, zq, q);
@@ -111,8 +88,8 @@ enum { cA, cB, ccw, cS0, cS1, cS2, ca0, ca2, cai, cFb, ck, cLf, cTm, cm1, calpha
 template <int K>
 __device__ __forceinline__ void diffuse(const double* __restrict__ lo, const double* __restrict__ up, int lane,
                                         const double (&tb)[K], double (&out)[K]) {
-  const double left = shfl_up1(tb[K - 1]);
-  const double right = shfl_dn1(tb[0]);
+  const double left = ebm_shfl_up1(tb[K - 1]);
+  const double right = ebm_shfl_dn1(tb[0]);
   // d[i] = T[j] - T[j-1] for the lane's cells, d[K] towards the next lane: each difference serves two cells
   double d[K + 1];
   d[0] = tb[0] - left;
@@ -142,7 +119,7 @@ __device__ __forceinline__ void tridiag(int lane, RowFn row, double (&rhs)[K]) {
       double jl_i, jd_i, ju_i;
       row(i, jl_i, jd_i, ju_i);
       const double P = (i == 0) ? jd_i : fma(jd_i, Pm1, -((jl_i * jup) * Pm2));
-      const double iw = Pm1 * rcp_nr(P);
+      const double iw = Pm1 * ebm_rcp(P);
       s[i] = jl_i * iw;                       // tq_i, turned into the spike below
       q[i] = ju_i * iw;
       rhs[i] = rhs[i] * iw;
@@ -163,13 +140,13 @@ __device__ __forceinline__ void tridiag(int lane, RowFn row, double (&rhs)[K]) {
     ga = -q[i] * ga;
   }
   // interface row of this lane:  A z_{l-1} + B z_l + C z_{l+1} = R, from the next lane's (al, be, ga)
-  const double nal = shfl_dn1(al), nbe = shfl_dn1(be), nga = shfl_dn1(ga);
+  const double nal = ebm_shfl_dn1(al), nbe = ebm_shfl_dn1(be), nga = ebm_shfl_dn1(ga);
   const double ql = (lane == 31) ? 0.0 : q[K - 1];
   double A = (lane == 0) ? 0.0 : s[K - 1];
   double C = -ql * nga;
   double R = fma(-ql, nal, rhs[K - 1]);
   {
-    const double ib = rcp_nr(fma(-ql, nbe, 1.0));
+    const double ib = ebm_rcp(fma(-ql, nbe, 1.0));
     A *= ib; C *= ib; R *= ib;
   }
   // parallel cyclic reduction, rows kept normalised (B = 1); out-of-range neighbours are identity rows
@@ -180,14 +157,14 @@ __device__ __forceinline__ void tridiag(int lane, RowFn row, double (&rhs)[K]) {
     const double Au = __shfl_up_sync(kFull, A, st), Cu = __shfl_up_sync(kFull, C, st), Ru = __shfl_up_sync(kFull, R, st);
     const double Ad = __shfl_down_sync(kFull, A, st), Cd = __shfl_down_sync(kFull, C, st), Rd = __shfl_down_sync(kFull, R, st);
     const double a_ = (lane >= st) ? A : 0.0, c_ = (lane + st < 32) ? C : 0.0;
-    const double ib = rcp_nr(fma(-a_, Cu, fma(-c_, Ad, 1.0)));
+    const double ib = ebm_rcp(fma(-a_, Cu, fma(-c_, Ad, 1.0)));
     const double Rn = fma(-a_, Ru, fma(-c_, Rd, R));
     A = -(a_ * Au) * ib;
     C = -(c_ * Cd) * ib;
     R = Rn * ib;
   }
   const double z = R;
-  const double zup = shfl_up1(z);              // every lane executes the shuffle (full mask)
+  const double zup = ebm_shfl_up1(z);              // every lane executes the shuffle (full mask)
   const double xL = (lane == 0) ? 0.0 : zup;
   double xn = z;
   rhs[K - 1] = z;
@@ -203,15 +180,14 @@ __device__ __forceinline__ void tridiag(int lane, RowFn row, double (&rhs)[K]) {
 __device__ __forceinline__ void store_cell(const MizKArgs& a, int j, long long msel, int year, int ti, int season,
                                            const double (&v)[EBM_MIZ_NVAR]) {
   const int nx = a.nx, nt = a.nt;
-  if (a.raw != nullptr && (!a.lastonly || year == a.dur - 1)) {
-    const long long nraw = a.lastonly ? (long long)nt : (long long)nt * a.dur;
-    const long long rawidx = a.lastonly ? (ti - 1) : ((long long)year * nt + ti - 1);
-    double* o = a.raw + ((msel * nraw + rawidx) * EBM_MIZ_NVAR) * (long long)nx + j;
+  if (a.raw != nullptr && (!a.lastonly || year == a.dur - 1)) {   // not ebm_raw_year: -70 to +11 instructions
+    double* o = a.raw + ebm_raw_offset(msel, ebm_nraw(nt, a.dur, a.lastonly), ebm_raw_slot(year, ti, nt, a.lastonly),
+                                       EBM_MIZ_NVAR, nx) + j;
 #pragma unroll
     for (int q = 0; q < EBM_MIZ_NVAR; ++q) o[(long long)q * nx] = v[q];
   }
   if (a.seasonal != nullptr) {
-    double* yr = a.seasonal + ((msel * a.dur + year) * 3) * (long long)EBM_MIZ_NVAR * nx + j;
+    double* yr = a.seasonal + ebm_seasonal_offset(msel, a.dur, year, 0, EBM_MIZ_NVAR, nx) + j;
     // the annual-mean slot doubles as the running sum of the year (annusol.raw -> crossmean, :556-559, :583-588)
     double* av = yr + 2LL * EBM_MIZ_NVAR * nx;
 #pragma unroll
@@ -248,7 +224,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
     for (int i = 0; i < K; ++i) {
       const int j = lane * K + i;
       double cu = 0.0, cl = 0.0;
-      if (j < nx) {
+      if (j < nx) {   // not a shared helper: every formulation tried reorders this kernel's code
         if (kind == 1) {   // generic flux-form stencil, infrastructure.jl:510-524
           cu = (j < nx - 1) ? a.g.mxxph[j] / a.g.diffx[j + 1] / a.g.phmmh[j] : 0.0;
           cl = (j > 0) ? a.g.mxxmh[j] / a.g.diffx[j] / a.g.phmmh[j] : 0.0;
@@ -286,7 +262,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
     c[cdt_Lf] = dt / pLf;                                                    // :139
     c[ctwoLf] = 2 * pLf;
     c[ctworl] = 2.0 * prl;
-    c[cinv_cw] = 1.0 / c[ccw]; c[cinv_Lf] = 1.0 / pLf; c[cinv_hmin] = rcp_nr(phmin);
+    c[cinv_cw] = 1.0 / c[ccw]; c[cinv_Lf] = 1.0 / pLf; c[cinv_hmin] = ebm_rcp(phmin);
     c[cc_r1] = 4.0 * prl; c[cc_r2] = 4.0 * prl * prl;                        // (D + 2 rl)^2 - D^2 = 4 rl D + 4 rl^2  (:91)
     c[cc_wl0] = -c[cm1] * c[cTm_m2];                                         // wlat = m1*Tw - m1*Tm^m2       (:71)
     c[ccBF] = c[cB] * pTm + c[cFb];
@@ -296,8 +272,8 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
   const double* cst = tabs.cst[warp];   // re-read after every STEP_FENCE: constants are CSE'd within a phase only
 #define CST(name) (cst[c##name])
 #define STEP_FENCE() asm volatile("" ::: "memory")
-  const bool constf = cst[cF0 + 1] == cst[cF0] && cst[cF0 + 2] == cst[cF0] && cst[cF0 + 6] == 0.0 &&
-                      cst[cF0 + 7] == 0.0 && cst[cF0 + 8] == 0.0 && cst[cF0 + 9] == 0.0;
+  const auto frow = [&](int r) { return cst[cF0 + r]; };
+  const bool constf = ebm_forcing_const(frow);
 
   // Ei, Ew and D are read and written once per step (outside the closure): they live in thread-private shared
   // memory [array][i][lane]; h, phi and the warm start T0 stay in registers
@@ -318,13 +294,13 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
     EI(i) = v ? a.Ei[o] : 0.0; EW(i) = v ? a.Ew[o] : 0.0; HH(i) = v ? a.h[o] : 0.0;
     DD(i) = v ? a.D[o] : 0.0; phi[i] = v ? a.phi[o] : 0.0; T0[i] = v ? a.T0[o] : 0.0;
     const double h0 = HH(i);
-    RHP(i) = sel(is_zero(h0), cst[cinv_hmin], rcp_nr(sel1(is_zero(h0), h0)));   // same expression as in the step
+    RHP(i) = sel(is_zero(h0), cst[cinv_hmin], ebm_rcp(sel1(is_zero(h0), h0)));   // same expression as in the step
   }
   double accT = 0.0, accE = 0.0, accP = 0.0;   // running hemispheric sums of the year (annual means are linear)
   unsigned icebits = 0u;
 
-  const bool sel_m = a.field_stride > 0 && (m % a.field_stride) == 0 && (a.seasonal != nullptr || a.raw != nullptr);
-  const long long msel = sel_m ? m / a.field_stride : 0;
+  const bool sel_m = ebm_field_selected(a, m) && (a.seasonal != nullptr || a.raw != nullptr);
+  const long long msel = sel_m ? ebm_field_row(a, m) : 0;
   long long iters_total = 0, fails_total = 0;
   const long long step_stop = a.step_limit > 0 ? (long long)a.step_limit : 0x7fffffffffffffffLL;
   const double tol = a.tol;
@@ -337,11 +313,9 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
       const double S1c = CST(S1) * __ldg(a.g.ctab + (ti - 1));                   // S1*cos(2*pi*t)
       double f = cst[cF0];
       if (!constf)
-        f = ebm_forcing_eval(cst[cF0], cst[cF0 + 1], cst[cF0 + 2], cst[cF0 + 3], cst[cF0 + 4], cst[cF0 + 6], cst[cF0 + 7],
-                             cst[cF0 + 8], cst[cF0 + 9],
-                             ebm_global_time((long long)(year + a.start_year) * nt + ti, nt));
+        f = ebm_forcing_at(frow, (long long)(year + a.start_year) * nt + ti, nt);
       const double fA = f - CST(A);
-      const int season = (ti == a.winter_inx) ? 0 : (ti == a.summer_inx) ? 1 : (ti == nt) ? 2 : -1;
+      const int season = ebm_season(a, ti, nt);
 
       // ---- temperatures and the closure's per-step constants (miz.jl:156-158, :33-60)
       double omTw[K], kb[K], c0[K];
@@ -350,7 +324,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
         const int s = i * 32 + lane;
         const double om = 1 - phi[i];
         const bool one = phi[i] == 1.0;
-        const double r_om = rcp_nr(sel1(one, om));                         // shared by water_temp and split_psiEw
+        const double r_om = ebm_rcp(sel1(one, om));                         // shared by water_temp and split_psiEw
         ROM(i) = r_om;
         const double ew = EW(i);
         // Ew / ((1-phi) cw) (:30); phi == 1: the IEEE quotient by +0 (NaN for Ew == 0 or NaN, else +-Inf)
@@ -389,7 +363,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
           g[i] = (T0[i] < CST(Tm)) ? phi[i] : 0.0;
           res[i] = (lane * K + i >= nx) ? 0.0 : res[i];
         }
-        const double gleft = shfl_up1(g[K - 1]), gright = shfl_dn1(g[0]);
+        const double gleft = ebm_shfl_up1(g[K - 1]), gright = ebm_shfl_dn1(g[0]);
         tridiag<K>(lane, [&](int i, double& jl, double& jd, double& ju) {
           const int s = i * 32 + lane;
           const double l = lo[s], u = up[s];
@@ -454,7 +428,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
         FORG Fvi[g] = c0[I] + common[g];                                               // :99-100 (ice)
         FORG Fvw[g] = fma(fma(-CST(a2), x2j[g], CST(a0)), S[g], fA) + common[g];       // (water)
         FORG wl[g] = fma(CST(m1), tw[g], CST(c_wl0));                                  // :71
-        FORG rD[g] = rcp_nr(sel1(noD[g], Do[g]));
+        FORG rD[g] = ebm_rcp(sel1(noD[g], Do[g]));
         FORG an[g] = sel0(noD[g], pho[g] * (rD[g] * rD[g]));                           // alpha * n
         FORG n[g] = an[g] * CST(inv_alpha);                                            // num :84-85
         FORG Flat[g] = sel0(noD[g], (pho[g] * ho[g]) * (wl[g] * CST(c_flat)) * rD[g]); // :104-105
@@ -474,7 +448,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
         FORG rDn[g] = fma(Dt[g], dt, Do[g]);                                           // :175
         FORG total[g] = n[g] + dn[g];
         FORG tz[g] = is_zero(total[g]);
-        FORG rt[g] = rcp_nr(sel1(tz[g], total[g]));
+        FORG rt[g] = ebm_rcp(sel1(tz[g], total[g]));
         FORG Dn[g] = sel0(tz[g], fma(n[g], rDn[g], dn[g] * CST(Dmin)) * rt[g]);        // average :131-132
         FORG Dn[g] = sel(Dn[g] > CST(Dmax), CST(Dmax), sel(Dn[g] < CST(Dmin), CST(Dmin), Dn[g]));   // clamp (NaN stays NaN) :177
         FORG Dn[g] = sel0(is_zero(Ei_n[g]), Dn[g]);                                    // :178
@@ -482,7 +456,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
         FORG rh[g] = rh[g] < 0.0 ? 0.0 : rh[g];                                        // :180
         FORG hn[g] = sel0(tz[g], fma(n[g], rh[g], dn[g] * CST(hmin)) * rt[g]);         // :181
         FORG hz[g] = is_zero(hn[g]);
-        FORG r_hn[g] = rcp_nr(sel1(hz[g], hn[g]));
+        FORG r_hn[g] = ebm_rcp(sel1(hz[g], hn[g]));
         FORG RHP(I) = sel(hz[g], CST(inv_hmin), r_hn[g]);                              // next step's 1/hp (:51)
         FORG ph[g] = sel0(hz[g], -Ei_n[g] * r_hn[g] * CST(inv_Lf));                    // concentration :75-76
         FORG { if (ph[g] > 1.0) ph[g] = 1.0; }                                         // :77
@@ -527,11 +501,8 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
         if (season == 2) {   // annual means: mean over the year of the hemispheric means (linear)
           dgT = accT / ntd; dgE = accE / ntd; dgP = accP / ntd;
         }
-        const double t0 = warp_sum(dgT), t1 = warp_sum(dgE), t2 = warp_sum(dgP), t3 = warp_min(dgX);
-        if (lane == 0) {
-          double* o = a.diag + ((m * a.dur + year) * 3 + season) * 4;
-          o[0] = t0; o[1] = t1; o[2] = 2.0 * kPi * t2; o[3] = (t3 > 1.5) ? 1.0 : t3;
-        }
+        const double t0 = ebm_warp_sum(dgT), t1 = ebm_warp_sum(dgE), t2 = ebm_warp_sum(dgP), t3 = ebm_warp_min(dgX);
+        if (lane == 0) ebm_store_diag(a.diag, m, a.dur, year, season, t0, t1, t2, t3);
       }
       if (ti == nt) { accT = accE = accP = 0.0; icebits = 0u; }
     }
@@ -546,8 +517,8 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) miz_fast_kernel(const MizKA
       const long long o = (long long)j * nmem + m;
       const double ei = EI(i), ew = EW(i), dd = DD(i);
       a.Ei[o] = ei; a.Ew[o] = ew; a.h[o] = HH(i); a.D[o] = dd; a.phi[o] = phi[i]; a.T0[o] = T0[i];
-      bad = bad || !(fabs(ei) < 1e300) || !(fabs(ew) < 1e300) || !(fabs(HH(i)) < 1e300) ||
-            !(fabs(dd) < 1e300) || !(fabs(phi[i]) < 1e300);
+      bad = bad || ebm_state_bad(ei) || ebm_state_bad(ew) || ebm_state_bad(HH(i)) || ebm_state_bad(dd) ||
+            ebm_state_bad(phi[i]);
     }
   }
   bad = __any_sync(kFull, bad);
@@ -575,7 +546,6 @@ int launch_k(const MizKArgs& a, cudaStream_t stream) {
 
 int ebm_launch_miz_fast(const MizKArgs& a, cudaStream_t stream) {
   if (a.nx < 3) { ebm_set_error("miz: nx must be >= 3"); return EBM_ERR_INVALID; }
-  if (a.single_ti > 0) return ebm_launch_miz_strict(a, stream);
   if (a.nx <= 64) return launch_k<2, 4>(a, stream);
   if (a.nx <= 128) return launch_k<4, 4>(a, stream);
   if (a.nx <= 192) return launch_k<6, 3>(a, stream);   // 3 resident CTAs per SM (168 registers): fastest measured

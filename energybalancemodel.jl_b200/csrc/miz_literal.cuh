@@ -18,9 +18,8 @@
 //   * there is no CTA barrier in the time loop and no shared-memory traffic between lanes: neighbour
 //     temperatures cross lanes with two shuffles per stencil evaluation, and the Newton convergence test is a
 //     warp vote, so every member takes exactly the iterations it needs (no lock-step across members).
-//   * the closure's linear system (tridiagonal, strictly diagonally dominant) is solved partitioned: each lane
-//     eliminates its K rows carrying a left spike, the 32 interface unknowns are solved by parallel cyclic
-//     reduction over shuffles (5 steps), each lane back-substitutes.
+//   * the closure's linear system (tridiagonal, strictly diagonally dominant) is solved by one lane, serial Thomas
+//     in the oracle's order, through shared memory.
 //   * geometry tables (x, x^2, trapezoid weights, stencil coefficients) are per-CTA shared memory laid out
 //     [cell-in-lane][lane] (bank-conflict free); member parameters are warp-uniform registers.
 //   * the insolation cos(2*pi*t) comes from a per-step table built on the host (same libm as the oracle).
@@ -32,8 +31,6 @@
 
 namespace {
 
-constexpr double kPi = 3.141592653589793;   // Float64(pi)
-constexpr unsigned kFull = 0xffffffffu;
 constexpr int kWarpsPerCta = 1;
 
 // Julia min(a, b): NaN-propagating (SURVEY Appendix C.6)
@@ -45,20 +42,6 @@ __device__ __forceinline__ double jl_min(double a, double b) {
 // Julia clamp(x, lo, hi) = ifelse(x > hi, hi, ifelse(x < lo, lo, x)); NaN passes through
 __device__ __forceinline__ double jl_clamp(double x, double lo, double hi) { return x > hi ? hi : (x < lo ? lo : x); }
 
-__device__ __forceinline__ double shfl_up1(double v) { return __shfl_up_sync(kFull, v, 1); }
-__device__ __forceinline__ double shfl_dn1(double v) { return __shfl_down_sync(kFull, v, 1); }
-
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(kFull, v, o);
-  return v;
-}
-__device__ __forceinline__ double warp_min(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(kFull, v, o));
-  return v;
-}
-
 struct MizPar {   // miz_paramset, src/infrastructure.jl:436-441
   double D, A, B, cw, S0, S1, S2, a0, a2, ai, Fb, k, Lf, Tm, m1, m2, alpha, rl, Dmin, Dmax, hmin, kappa;
 };
@@ -67,8 +50,7 @@ struct MizPar {   // miz_paramset, src/infrastructure.jl:436-441
 template <int K>
 struct MizTabs {
   double x[K * 32], x2[K * 32], wts[K * 32];
-  // fast flavour: diffusion_j = D*(cu_j*(T[j+1]-T[j]) - cl_j*(T[j]-T[j-1]))
-  double cu[K * 32], cl[K * 32];
+  double cu[K * 32], cl[K * 32];   // stencil coefficient towards j+1 / j-1
   // literal stencils: generic (mxxph, mxxmh, phmmh, diffx[j+1], diffx[j]) / identity (lam_hi, lam_lo)
   double mxxph[K * 32], mxxmh[K * 32], phmmh[K * 32], dxp[K * 32], dxm[K * 32];
   double scratch[6][K * 32];   // serial Thomas: jl, jd, ju, rhs, w, y
@@ -84,13 +66,13 @@ struct MizMember {
 };
 
 // ---- diffusion of a temperature profile held K cells per lane (increment only: D * nabla^2 T) -----------------
-// tb[i] are the lane's cells; neighbours come from the adjacent lanes.  Zero flux at both ends: the stencil
-// coefficient towards a missing neighbour is 0 (fast) / the difference is 0 (literal, infrastructure.jl:522).
+// tb[i] are the lane's cells; neighbours come from the adjacent lanes.  Zero flux at both ends: the difference
+// (generic stencil, infrastructure.jl:522) / the get_diffop coefficient towards a missing neighbour is 0.
 template <int K>
 __device__ __forceinline__ void miz_diffusion(const MizTabs<K>& tb_, const MizPar& p, int kind, int nx, int lane,
                                               const double (&tb)[K], double (&out)[K]) {
-  const double left = shfl_up1(tb[K - 1]);    // cell j-1 of my first cell (garbage for lane 0: masked)
-  const double right = shfl_dn1(tb[0]);       // cell j+1 of my last cell
+  const double left = ebm_shfl_up1(tb[K - 1]);    // cell j-1 of my first cell (garbage for lane 0: masked)
+  const double right = ebm_shfl_dn1(tb[0]);       // cell j+1 of my last cell
 #pragma unroll
   for (int i = 0; i < K; ++i) {
     const int s = i * 32 + lane;
@@ -115,13 +97,11 @@ __device__ __forceinline__ void miz_diffusion(const MizTabs<K>& tb_, const MizPa
   }
 }
 
-// ---- tridiagonal solve across the warp: rows (jl, jd, ju) x = rhs, K rows per lane --------------------------------
-// On return rhs holds the solution.  Fast flavour: partitioned elimination + PCR on the 32 interface unknowns.
+// ---- tridiagonal solve: rows (jl, jd, ju) x = rhs, K rows per lane ------------------------------------------------
+// On return rhs holds the solution.  Literal Thomas in the oracle's order (one lane), through shared memory.
 template <int K>
-__device__ __forceinline__ void miz_tridiag(MizTabs<K>& tabs, int warp, int nx, int lane, const double (&jl)[K],
+__device__ __forceinline__ void miz_tridiag(MizTabs<K>& tabs, int nx, int lane, const double (&jl)[K],
                                             const double (&jd)[K], const double (&ju)[K], double (&rhs)[K]) {
-  (void)warp;
-  // literal Thomas in the oracle's order (one lane), through shared memory
   double* sl = tabs.scratch[0]; double* sd = tabs.scratch[1]; double* su = tabs.scratch[2];
   double* sr = tabs.scratch[3]; double* w = tabs.scratch[4]; double* y = tabs.scratch[5];
 #pragma unroll
@@ -156,7 +136,7 @@ __device__ __forceinline__ void miz_tridiag(MizTabs<K>& tabs, int warp, int nx, 
 // so a semi-smooth Newton iteration stopped at max|res| <= tol (reference: abstol 1e-8) finds the root the
 // reference's TrustRegion solver is asked for.  Returns the number of Newton iterations; *fail if not converged.
 template <int K>
-__device__ __forceinline__ int miz_solveTi(MizTabs<K>& tabs, const MizPar& p, int kind, int nx, int lane, int warp,
+__device__ __forceinline__ int miz_solveTi(MizTabs<K>& tabs, const MizPar& p, int kind, int nx, int lane,
                                            double f, double c2pt, const double (&h)[K], const double (&Tw)[K],
                                            const double (&phi)[K], double (&T0)[K], double (&Ti)[K], double tol,
                                            int maxit, int* fail) {
@@ -201,7 +181,7 @@ __device__ __forceinline__ int miz_solveTi(MizTabs<K>& tabs, const MizPar& p, in
     double g[K], jl[K], jd[K], ju[K];
 #pragma unroll
     for (int i = 0; i < K; ++i) g[i] = (T0[i] < p.Tm) ? phi[i] : 0.0;
-    const double gleft = shfl_up1(g[K - 1]), gright = shfl_dn1(g[0]);
+    const double gleft = ebm_shfl_up1(g[K - 1]), gright = ebm_shfl_dn1(g[0]);
 #pragma unroll
     for (int i = 0; i < K; ++i) {
       const int s = i * 32 + lane;
@@ -224,7 +204,7 @@ __device__ __forceinline__ int miz_solveTi(MizTabs<K>& tabs, const MizPar& p, in
       ju[i] = (j < nx - 1) ? up * gp : 0.0;
       res[i] = (j < nx) ? -res[i] : 0.0;
     }
-    miz_tridiag<K>(tabs, warp, nx, lane, jl, jd, ju, res);
+    miz_tridiag<K>(tabs, nx, lane, jl, jd, ju, res);
 #pragma unroll
     for (int i = 0; i < K; ++i) T0[i] += res[i];
     ++it;
@@ -243,10 +223,11 @@ template <int K>
 __device__ __forceinline__ void miz_store_fields(const MizKArgs& a, int lane, long long msel, int year, int ti,
                                                  int season, const double (&v)[EBM_MIZ_NVAR][K]) {
   const int nx = a.nx, nt = a.nt;
-  if (a.raw != nullptr && (a.single_ti > 0 || !a.lastonly || year == a.dur - 1)) {
-    const long long nraw = a.single_ti > 0 ? 1 : (a.lastonly ? (long long)nt : (long long)nt * a.dur);
-    const long long rawidx = a.single_ti > 0 ? 0 : (a.lastonly ? (ti - 1) : ((long long)year * nt + ti - 1));
-    double* o = a.raw + ((msel * nraw + rawidx) * EBM_MIZ_NVAR) * (long long)nx;
+  // the one step of ebm_miz_step (single_ti) has one raw slot
+  if (a.raw != nullptr && (a.single_ti > 0 || ebm_raw_year(year, a.dur, a.lastonly))) {
+    const long long nraw = a.single_ti > 0 ? 1 : ebm_nraw(nt, a.dur, a.lastonly);
+    const long long rawidx = a.single_ti > 0 ? 0 : ebm_raw_slot(year, ti, nt, a.lastonly);
+    double* o = a.raw + ebm_raw_offset(msel, nraw, rawidx, EBM_MIZ_NVAR, nx);
 #pragma unroll
     for (int q = 0; q < EBM_MIZ_NVAR; ++q)
 #pragma unroll
@@ -256,7 +237,7 @@ __device__ __forceinline__ void miz_store_fields(const MizKArgs& a, int lane, lo
       }
   }
   if (a.seasonal != nullptr) {
-    double* yr = a.seasonal + ((msel * a.dur + year) * 3) * (long long)EBM_MIZ_NVAR * nx;
+    double* yr = a.seasonal + ebm_seasonal_offset(msel, a.dur, year, 0, EBM_MIZ_NVAR, nx);
     // the annual-mean slot doubles as the running sum of the year (annusol.raw -> crossmean, :556-559, :583-588)
     double* av = yr + 2LL * EBM_MIZ_NVAR * nx;
 #pragma unroll
@@ -320,7 +301,8 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) miz_warp_kernel(const MizKA
   double fr[EBM_NFORCING];
 #pragma unroll
   for (int r = 0; r < EBM_NFORCING; ++r) fr[r] = (a.single_ti > 0) ? 0.0 : a.forc[(long long)r * nmem + m];
-  const bool constf = fr[1] == fr[0] && fr[2] == fr[0] && fr[6] == 0.0 && fr[7] == 0.0 && fr[8] == 0.0 && fr[9] == 0.0;
+  const auto frow = [&](int r) { return fr[r]; };
+  const bool constf = ebm_forcing_const(frow);
 
   const double dt = 1.0 / nt;
   const double Tm_m2 = pow(p.Tm, p.m2);                                     // wlat :71 -- `Tm^m2` binds to Tm (sic)
@@ -338,8 +320,8 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) miz_warp_kernel(const MizKA
   s.accT = s.accE = s.accP = 0.0;
   s.icebits = 0u;
 
-  const bool sel = a.field_stride > 0 && (m % a.field_stride) == 0 && (a.seasonal != nullptr || a.raw != nullptr);
-  const long long msel = sel ? m / a.field_stride : 0;
+  const bool sel = ebm_field_selected(a, m) && (a.seasonal != nullptr || a.raw != nullptr);
+  const long long msel = sel ? ebm_field_row(a, m) : 0;
   long long iters_total = 0, fails_total = 0;
 
   const int ti_first = a.single_ti > 0 ? a.single_ti : 1;
@@ -353,9 +335,8 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) miz_warp_kernel(const MizKA
       double f = fr[0];
       if (a.single_ti > 0) f = a.single_f;
       else if (!constf)
-        f = ebm_forcing_eval(fr[0], fr[1], fr[2], fr[3], fr[4], fr[6], fr[7], fr[8], fr[9],
-                             ebm_global_time((long long)(year + a.start_year) * nt + ti, nt));
-      const int season = (ti == a.winter_inx) ? 0 : (ti == a.summer_inx) ? 1 : (ti == nt) ? 2 : -1;
+        f = ebm_forcing_at(frow, (long long)(year + a.start_year) * nt + ti, nt);
+      const int season = ebm_season(a, ti, nt);
 
       // ---- temperatures (miz.jl:156-158)
       double Tw[K], Ti[K];
@@ -365,7 +346,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) miz_warp_kernel(const MizKA
         Tw[i] = (v != v) ? 0.0 : v;                                         // :157
       }
       int fail = 0;
-      iters_total += miz_solveTi<K>(tabs, p, kind, nx, lane, warp, f, c2pt, s.h, Tw, s.phi, s.T0, Ti, a.tol, a.maxit, &fail);
+      iters_total += miz_solveTi<K>(tabs, p, kind, nx, lane, f, c2pt, s.h, Tw, s.phi, s.T0, Ti, a.tol, a.maxit, &fail);
       fails_total += fail;
 
       // ---- fluxes (:160-164)
@@ -463,11 +444,8 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) miz_warp_kernel(const MizKA
         if (season == 2) {   // annual means: mean over the year of the hemispheric means (linear)
           dgT = s.accT / (double)nt; dgE = s.accE / (double)nt; dgP = s.accP / (double)nt;
         }
-        const double t0 = warp_sum(dgT), t1 = warp_sum(dgE), t2 = warp_sum(dgP), t3 = warp_min(dgX);
-        if (lane == 0) {
-          double* o = a.diag + ((m * a.dur + year) * 3 + season) * 4;
-          o[0] = t0; o[1] = t1; o[2] = 2.0 * kPi * t2; o[3] = (t3 > 1.5) ? 1.0 : t3;
-        }
+        const double t0 = ebm_warp_sum(dgT), t1 = ebm_warp_sum(dgE), t2 = ebm_warp_sum(dgP), t3 = ebm_warp_min(dgX);
+        if (lane == 0) ebm_store_diag(a.diag, m, a.dur, year, season, t0, t1, t2, t3);
       }
       if (ti == nt) { s.accT = s.accE = s.accP = 0.0; s.icebits = 0u; }
     }
@@ -481,8 +459,8 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) miz_warp_kernel(const MizKA
     if (j < nx) {
       const long long o = (long long)j * nmem + m;
       a.Ei[o] = s.Ei[i]; a.Ew[o] = s.Ew[i]; a.h[o] = s.h[i]; a.D[o] = s.D[i]; a.phi[o] = s.phi[i]; a.T0[o] = s.T0[i];
-      bad = bad || !(fabs(s.Ei[i]) < 1e300) || !(fabs(s.Ew[i]) < 1e300) || !(fabs(s.h[i]) < 1e300) ||
-            !(fabs(s.D[i]) < 1e300) || !(fabs(s.phi[i]) < 1e300);
+      bad = bad || ebm_state_bad(s.Ei[i]) || ebm_state_bad(s.Ew[i]) || ebm_state_bad(s.h[i]) || ebm_state_bad(s.D[i]) ||
+            ebm_state_bad(s.phi[i]);
     }
   }
   bad = __any_sync(kFull, bad);

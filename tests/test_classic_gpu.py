@@ -55,8 +55,9 @@ def test_single_step_bitwise():
 
 
 def test_strict_kernel_bitwise_one_year():
-    """C1a with the literal-arithmetic kernel: every step of E, T, h and the final Tg bit-identical."""
-    st = ebm.SpaceTime(100, 2000, 1)
+    """C1a with the literal-arithmetic kernel, run for two years: every step of E, T, h (the raw slots of both years)
+    and the final Tg bit-identical."""
+    st = ebm.SpaceTime(100, 2000, 2)
     par, f, init = _par(), ebm.Forcing(0.0), warm_init(100)
     o = oracle_classic(st, [f], [par], [init], lastonly=False, raw=True, seasonal=True)
     r = ebm.integrate_ensemble("Classic", st, [f], [par], [init], lastonly=False, field_stride=1, strict=True)
@@ -106,13 +107,17 @@ def _ensemble(nmem, nx):
     return forcings, pars, inits
 
 
-@pytest.mark.parametrize("nmem,nx,nt", [(70, 100, 2000), (33, 60, 1000), (5, 37, 500), (40, 180, 2000)])
-def test_ensemble_diag_fields_and_state(nmem, nx, nt):
+@pytest.mark.parametrize("nmem,nx,nt,lastonly", [
+    pytest.param(70, 100, 2000, True, id="70-100-2000"), pytest.param(33, 60, 1000, True, id="33-60-1000"),
+    pytest.param(5, 37, 500, True, id="5-37-500"), pytest.param(40, 180, 2000, True, id="40-180-2000"),
+    # raw output of every year (8-band and 16-band grids)
+    pytest.param(8, 60, 1000, False, id="8-60-1000-all-years"), pytest.param(4, 180, 2000, False, id="4-180-2000-all-years")])
+def test_ensemble_diag_fields_and_state(nmem, nx, nt, lastonly):
     """Ragged member counts / other grids: L0 diagnostics, L1/L2 fields of strided members, final state."""
     st = ebm.SpaceTime(nx, nt, 3)
     forcings, pars, inits = _ensemble(nmem, nx)
-    o = oracle_classic(st, forcings, pars, inits, lastonly=True, raw=True, seasonal=True)
-    r = ebm.integrate_ensemble("Classic", st, forcings, pars, inits, field_stride=3)
+    o = oracle_classic(st, forcings, pars, inits, lastonly=lastonly, raw=True, seasonal=True)
+    r = ebm.integrate_ensemble("Classic", st, forcings, pars, inits, field_stride=3, lastonly=lastonly)
     assert r.flags.max() == 0
     # E integrates cg_tau*Tg = 9800*Tg (classic.jl:48): a rounding difference of 1e-13 in the ghost-layer solve is
     # 1e-9 in the tendency.  At the BASELINE grid (nx = 100) everything stays under 1e-9; the finer 180-cell grid
@@ -143,10 +148,11 @@ def test_ramp_forcing_and_chained_launches():
     pars = [_par()] * 3
     inits = [warm_init(100), cold_init(100), warm_init(100)]
     o = oracle_classic(st, forcings, pars, inits, seasonal=True)
-    a = ebm.integrate_ensemble("Classic", st, forcings, pars, inits, field_stride=1, want_raw=False)
-    b = ebm.integrate_ensemble("Classic", st, forcings, pars, inits, field_stride=1, want_raw=False, years_per_launch=2)
+    a = ebm.integrate_ensemble("Classic", st, forcings, pars, inits, field_stride=1, lastonly=False)
+    b = ebm.integrate_ensemble("Classic", st, forcings, pars, inits, field_stride=1, lastonly=False, years_per_launch=2)
     assert rel_err(a.seasonal, o["seasonal"]).max() < TOL
     assert np.array_equal(a.final["E"], b.final["E"]) and np.array_equal(a.final["Tg"], b.final["Tg"])
+    assert a.raw.shape[1] == 6 * 2000 and np.array_equal(a.raw, b.raw)
     assert np.array_equal(np.nan_to_num(a.seasonal), np.nan_to_num(b.seasonal))
     assert np.array_equal(a.diag, b.diag)
 
@@ -367,17 +373,18 @@ def test_sixteen_band_table_driven_instance(nx):
     assert_close(r.diag[..., :2], oracle_diag_classic(o["seasonal"], st.x)[..., :2], tol, "diag")
 
 
-@pytest.mark.parametrize("nx", [230, 250])
-def test_band_kernel_large_grids(nx):
+@pytest.mark.parametrize("nx,lastonly", [pytest.param(230, True, id="230"), pytest.param(250, True, id="250"),
+                                         pytest.param(250, False, id="250-all-years")])   # raw output of both years
+def test_band_kernel_large_grids(nx, lastonly):
     """208 < nx <= 256: the band kernel (16 cells per band, 16 members per CTA).  nx = 230 needs 15 bands -- an odd
     count, which the launcher pads to whole warps (ADVICE r1: no thread may shadow another thread's band)."""
-    nmem = 20
+    nmem = 20 if lastonly else 5
     st = ebm.SpaceTime(nx, 2000, 2)
     forcings = [ebm.Forcing(-8.0 + 16.0 * m / (nmem - 1)) for m in range(nmem)]
     pars = [_par(B=2.0 + 0.05 * (m % 4)) for m in range(nmem)]
     inits = [warm_init(nx) if m % 2 == 0 else cold_init(nx) for m in range(nmem)]
-    o = oracle_classic(st, forcings, pars, inits, raw=True, seasonal=True)
-    r = ebm.integrate_ensemble("Classic", st, forcings, pars, inits, field_stride=4)
+    o = oracle_classic(st, forcings, pars, inits, lastonly=lastonly, raw=True, seasonal=True)
+    r = ebm.integrate_ensemble("Classic", st, forcings, pars, inits, field_stride=4, lastonly=lastonly)
     assert r.flags.max() == 0
     tol = 2e-8                                     # finer grids: see test_ensemble_diag_fields_and_state
     assert_close(r.final["E"], o["E"], tol, "final E")
